@@ -19,6 +19,9 @@ with the fp32 forward; single-pass bf16 does not -- DESIGN.md section 3); same k
   parity     (N = 1) max-abs / raw argmax agreement of the device output against the CPU baseline leg's output
   --impl reference   the reference's CPU forward (NumPy restatement = what Chainer's CPU backend executes; Chainer
              itself is not installable offline), ALL host cores, on a bounded sample of the workload
+  --dump-outputs DIR writes DIR/log_likelihoods.npy: float32 rows of the device-resident leg's (N, 1909) output after
+             its last timed step -- all of them, or a fixed seeded sample of DUMP_ROWS when N is larger -- so that two
+             builds run with the same arguments (same seeded inputs and weights) can be compared output for output
 
 The product arm builds its workload, weights and transform through the package only (nnacousticmodeling_b200.synth,
 Network.init_params, loadKaldiFeatureTransform); oracle/ is imported by the cpu_baseline / reference legs alone.
@@ -48,6 +51,7 @@ N_CLASSES = 1909
 TRAIN_UTTS, TRAIN_FRAMES = 3696, 1124823
 TEST_UTTS = 1344
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+DUMP_ROWS = 8192  # x 1909 float32 = 62.5 MB, within the 64 MB that --dump-outputs may write
 
 WORKLOADS = {
     # name: network, i-vector dim, units, layers, set, algorithmic flop/frame (SURVEY 8d)
@@ -361,6 +365,13 @@ class Bench:
                                      ivectors=self.ivp, device=self.local, head=self.head)
 
 
+def dump_rows(n):
+    """Output rows written by --dump-outputs: every row, or the same seeded sample of DUMP_ROWS rows on every run."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
 def timed_device(torch, fn, steps, barrier):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
@@ -525,6 +536,10 @@ def run_ours(args):
     prof, ops.PROFILE = ops.PROFILE, None
     launches = sum(ops.LAUNCHES.values()) - launches0
     value = world * n / (dev_ms * 1e-3)
+    # taken now: the legs below write other results into out_dev
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = b.out_dev[torch.from_numpy(dump_rows(n)).to(dev)].cpu().numpy()
     kern = kernel_table(prof, steps)
     roof = roofline_block(kern, peaks, args.workload, steps)
 
@@ -623,6 +638,9 @@ def run_ours(args):
     elif rank == 0:
         line["cpu_baseline"] = None
     if rank == 0:
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "log_likelihoods.npy"), dumped)
         emit(line)
     dist_util.finalize()
     return 0
@@ -730,7 +748,14 @@ def main():
     ap.add_argument("--no-cli", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end leg (profiling runs under ncu only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the device-resident leg's output of its last timed step to DIR/log_likelihoods.npy "
+                         f"(float32; a fixed seeded sample of {DUMP_ROWS} rows when the set is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the output of the device path: --impl ours only")
     if args.cpu_sample is None:
         # the cpu_baseline leg runs once (~10-30 s); the reference arm repeats its sample steps + warmup times
         args.cpu_sample = 65536 if args.impl == "reference" else 262144
