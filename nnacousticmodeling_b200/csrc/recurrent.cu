@@ -644,11 +644,12 @@ static size_t rnn_smem_bytes(const RnnCfg& c, int hidden, int cell) {
          8 * (1 + 2 * c.s) + 16 + static_cast<size_t>(c.s) * (c.nb + base_smem + 1) * 4 + 1024;
 }
 
-// The instance used for (hidden, slots per stream, precision), or nullptr.
-static const RnnCfg* rnn_pick_cfg(int cell, int hidden, int nb, int nsplit) {
+// The instance used for (hidden, slots per stream, precision), or nullptr.  single_stream: only one-stream instances
+// qualify (the descriptor was planned for the multicast kernel, which runs one stream, but carried state rules it out).
+static const RnnCfg* rnn_pick_cfg(int cell, int hidden, int nb, int nsplit, bool single_stream = false) {
   const int kbt = hidden / 64;
   // the opt-in cluster experiment replaces the single-stream instance
-  const bool single = (4 * hidden) % 128 == 0 && rnn_cluster_groups(cell, hidden, nb, nsplit) > 0;
+  const bool single = single_stream || ((4 * hidden) % 128 == 0 && rnn_cluster_groups(cell, hidden, nb, nsplit) > 0);
   const RnnCfg* list = cell == NNAM_CELL_PEEPHOLE ? kPeepCfgs : kRnnCfgs;
   const size_t n_list = cell == NNAM_CELL_PEEPHOLE ? sizeof(kPeepCfgs) / sizeof(RnnCfg) : sizeof(kRnnCfgs) / sizeof(RnnCfg);
   for (size_t i = 0; i < n_list; ++i) {
@@ -737,7 +738,11 @@ int rnn_seq(const NnamRnnDesc* d, cudaStream_t stream) {
                (d->n_dirs == 2 && (reinterpret_cast<uintptr_t>(d->gx[1]) & 31))))
     return set_error(NNAM_ERR_ARG, "rnn: 128 slots per batch need 32-byte aligned gx / h / exchange buffers and "
                      "gx_ld, h_ld multiples of 16 (256-bit accesses)");
-  const RnnCfg* cfg = wide ? &kWideCfg : rnn_pick_cfg(d->cell, H, d->batch, d->nsplit);
+  // nnam_rnn_plan promises one stream wherever the multicast kernel applies; with carried state that kernel is ruled out
+  // and the counter-based kernel must run the same single-stream schedule
+  const bool carried = d->h0_hi || d->c0 || d->c_out;
+  const bool mc_planned = !wide && rnn_mc_groups(d->cell, H, d->batch, d->nsplit) > 0;
+  const RnnCfg* cfg = wide ? &kWideCfg : rnn_pick_cfg(d->cell, H, d->batch, d->nsplit, mc_planned && carried);
   if (!cfg)
     return set_error(NNAM_ERR_UNSUPPORTED,
                      "rnn: no kernel instance holds the lateral weights of H=%d in shared memory with %d slots per "
@@ -747,10 +752,9 @@ int rnn_seq(const NnamRnnDesc* d, cudaStream_t stream) {
   const int max_groups = sm_count() / G;
   if (d->n_groups < 1 || d->n_groups > max_groups)
     return set_error(NNAM_ERR_ARG, "rnn: n_groups %d outside [1, %d]", d->n_groups, max_groups);
-  const bool mc_plan = !wide && !d->h0_hi && !d->c0 && !d->c_out && rnn_mc_groups(d->cell, H, d->batch, d->nsplit) > 0;
-  if (d->streams != (mc_plan ? 1 : cfg->s))
+  if (d->streams != (mc_planned ? 1 : cfg->s))
     return set_error(NNAM_ERR_ARG, "rnn: descriptor built for %d streams per group, this configuration runs %d "
-                     "(ask nnam_rnn_plan)", d->streams, cfg->s);
+                     "(ask nnam_rnn_plan)", d->streams, mc_planned ? 1 : cfg->s);
   // experimental DSMEM variant: groups are independent clusters (no carried state through this path)
   const bool use_cluster = m_rows == 128 && cfg->s == 1 && !d->h0_hi && !d->c0 && !d->c_out &&
                            rnn_cluster_groups(d->cell, H, d->batch, d->nsplit) > 0;
