@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define NNAM_ABI_VERSION 3
+#define NNAM_ABI_VERSION 4
 
 /* error codes */
 #define NNAM_OK 0
@@ -141,6 +141,20 @@ int nnam_head_f16(const float* const* logits_host, const float* weights_host, in
                   float prior_scale, int final_normalize, void* out16, long long ld16, float* row_ref, long long rows,
                   int n_classes, const int* out_row_map, void* stream);
 
+/* nnam_head_scatter scored against frame targets instead of writing rows: with y[q] the row nnam_head_scatter would write
+ * to output row q (same arguments, same kernel choice, the same device code),
+ *   nll[q]  = -y[q][targets[q]], or 0 when targets[q] == -1 (Chainer's ignore_label)
+ *   pred[q] = argmax_c y[q][c], the lowest column on ties
+ * An out_row_map entry -1 drops the row (nothing is written) and -2 - q writes nll[q] = 0, pred[q] = -1 (the zero rows of
+ * quirk Q4 are no network output).  targets: int[rows_out] in [-1, n_classes) (the host validates them), nll:
+ * float[rows_out], pred: int[rows_out].  8 B per row leave the kernel instead of 4 * n_classes.
+ * Replaces what training reports per frame (recalled from Chainer upstream, †): F.softmax_cross_entropy (the mean of
+ * nll over targets != -1) and F.accuracy, behind L.Classifier as train.py uses it (SURVEY section 2, rows 11-13).  */
+int nnam_head_score(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in,
+                    int pre_normalize, const float* rpl_w, const float* rpl_b, const float* rpl_lb, const float* prior,
+                    float prior_scale, int final_normalize, const int* targets, float* nll, int* pred, long long rows,
+                    int n_classes, const int* out_row_map, void* stream);
+
 /* K2 + K4 fused for ONE net without RPL: out = log_softmax(A . W^T + bias - prior_scale * prior), i.e. the output
  * L.Linear (chainer_networks.py:21-22, 61-62, ...) followed by `y - logsum(y, axis=1)` (predict_folds.py:57,88) or by
  * `y = y - ap; y - logsum(y)` (evaluateModelForTest.py:75-77,110-112), without the float32 logits ever going to HBM:
@@ -153,6 +167,16 @@ int nnam_linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, co
                            long long ldw, const float* bias, const float* prior, float prior_scale, float* out,
                            long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map,
                            int M, int N, int K, int nsplit, int elem, void* stream);
+
+/* nnam_linear_logsoftmax scored against frame targets instead of writing rows: nll / pred / targets and the row map as
+ * in nnam_head_score, y the float32 rows nnam_linear_logsoftmax writes with the same operands (the argmax is taken over
+ * those written values, not over the logits: rounding bias - lse per column can reorder two near-tied columns).
+ * Replaces (recalled from Chainer upstream, †) F.softmax_cross_entropy and F.accuracy behind L.Classifier, as used by
+ * train.py, for a net whose output layer runs fused with its head.  */
+int nnam_linear_logsoftmax_score(const void* a_hi, const void* a_lo, long long lda, const void* w_hi, const void* w_lo,
+                                 long long ldw, const float* bias, const float* prior, float prior_scale,
+                                 const int* targets, float* nll, int* pred, const int* out_row_map, int M, int N, int K,
+                                 int nsplit, int elem, void* stream);
 
 /* HOST function (no CUDA): dst_host[q][c] = float(src16_host[r][c]) + row_ref_host[r] for r < rows, c < cols, with
  * q = r, or q = dst_rows_host[r] when that map is given (the recurrent path ships a subset of utterances as one

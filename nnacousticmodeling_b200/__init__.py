@@ -2,6 +2,7 @@
 
 Feature matrix (+ offsets, i-vectors, Kaldi feature transform) -> per-frame pdf log-likelihoods,
 behind the reference's Python surface (get_nn / model specs / predict / evaluateModelTestTri),
+and their scores against frame targets (``score``: cross-entropy and frame accuracy, reduced on the device),
 computed by hand-written sm_100a CUDA kernels in ``libnnam_b200.so`` (C ABI: include/nnam_b200.h).
 There is no CPU fallback.
 """
@@ -17,6 +18,7 @@ from .features import (  # noqa: F401
 from .engine import empty_pinned, partition_frames, partition_utterances  # noqa: F401
 from .engine import HeadSpec  # noqa: F401
 from .predict import predict  # noqa: F401
+from .score import FrameScore, score  # noqa: F401
 from . import evaluate  # noqa: F401
 from .evaluate import NNWithRPL, evaluateModelTestTri  # noqa: F401
 

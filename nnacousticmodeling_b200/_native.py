@@ -18,7 +18,7 @@ SOURCES = ["api.cu", "gemm.cu", "gemm_head.cu", "splice.cu", "head.cu", "recurre
            "host_widen.cpp"]  # .cpp = host-only code, compiled with the host C++ compiler
 # measured dead end kept for reference (DSMEM all-gather recurrence); NNAM_WITH_CLUSTER_EXPERIMENT=1 builds it in
 EXPERIMENTAL_SOURCES = ["experimental/recurrent_cluster.cu"]
-ABI_VERSION = 3
+ABI_VERSION = 4
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared",
@@ -114,6 +114,13 @@ _SIGNATURES = {
     "nnam_linear_logsoftmax": (c_int, [c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p,
                                        c_float, c_void_p, c_longlong, c_void_p, c_longlong, c_void_p, c_void_p, c_int,
                                        c_int, c_int, c_int, c_int, c_void_p]),
+    # scoring forms of nnam_head_scatter / nnam_linear_logsoftmax (Chainer's softmax_cross_entropy + accuracy, †)
+    "nnam_head_score": (c_int, [POINTER(c_void_p), POINTER(c_float), c_int, c_longlong, c_int, c_void_p, c_void_p,
+                                c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_void_p, c_longlong, c_int,
+                                c_void_p, c_void_p]),
+    "nnam_linear_logsoftmax_score": (c_int, [c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p,
+                                             c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                             c_int, c_int, c_int, c_void_p]),
     "nnam_widen_f16_host": (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_longlong, c_int,
                                     c_int]),
     "nnam_gather_transform": (c_int, [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p,

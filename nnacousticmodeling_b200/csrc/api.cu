@@ -82,7 +82,7 @@ int convert_f32(const float* src, long long rows, int cols, long long lds, void*
 int head(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in, int pre_normalize,
          const float* rpl_w, const float* rpl_b, const float* rpl_lb, const float* prior, float prior_scale,
          int final_normalize, float* out, long long ld_out, long long rows, int n_classes, const int* out_row_map,
-         void* out16, long long ld16, float* row_ref, cudaStream_t stream);
+         void* out16, long long ld16, float* row_ref, const int* targets, float* nll, int* pred, cudaStream_t stream);
 int gather_transform(const float* x, long long n_src, int dim, const float* add_shift, const float* rescale,
                      const float* ivec, int ivec_dim, const int* row_map, long long n_rows, void* out_hi, void* out_lo,
                      long long ldo, int out_kind, cudaStream_t stream);
@@ -132,7 +132,18 @@ int nnam_linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, co
                            long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map,
                            int M, int N, int K, int nsplit, int elem, void* stream) {
   return nnam::linear_logsoftmax(a_hi, a_lo, lda, w_hi, w_lo, ldw, bias, prior, prior_scale, out, ld_out, out16, ld16,
-                                 row_ref, out_row_map, M, N, K, nsplit, elem, static_cast<cudaStream_t>(stream));
+                                 row_ref, out_row_map, nullptr, nullptr, nullptr, M, N, K, nsplit, elem,
+                                 static_cast<cudaStream_t>(stream));
+}
+
+int nnam_linear_logsoftmax_score(const void* a_hi, const void* a_lo, long long lda, const void* w_hi, const void* w_lo,
+                                 long long ldw, const float* bias, const float* prior, float prior_scale,
+                                 const int* targets, float* nll, int* pred, const int* out_row_map, int M, int N, int K,
+                                 int nsplit, int elem, void* stream) {
+  if (nll == nullptr) return nnam::set_error(NNAM_ERR_ARG, "linear_logsoftmax_score: nll is NULL");
+  return nnam::linear_logsoftmax(a_hi, a_lo, lda, w_hi, w_lo, ldw, bias, prior, prior_scale, nullptr, 0, nullptr, 0,
+                                 nullptr, out_row_map, targets, nll, pred, M, N, K, nsplit, elem,
+                                 static_cast<cudaStream_t>(stream));
 }
 
 int nnam_head(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in,
@@ -140,8 +151,8 @@ int nnam_head(const float* const* logits_host, const float* weights_host, int n_
               float prior_scale, int final_normalize, float* out, long long ld_out, long long rows, int n_classes,
               void* stream) {
   return nnam::head(logits_host, weights_host, n_inputs, ld_in, pre_normalize, rpl_w, rpl_b, rpl_lb, prior,
-                    prior_scale, final_normalize, out, ld_out, rows, n_classes, nullptr, nullptr, 0, nullptr,
-                    static_cast<cudaStream_t>(stream));
+                    prior_scale, final_normalize, out, ld_out, rows, n_classes, nullptr, nullptr, 0, nullptr, nullptr,
+                    nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int nnam_head_scatter(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in,
@@ -149,8 +160,8 @@ int nnam_head_scatter(const float* const* logits_host, const float* weights_host
                       const float* prior, float prior_scale, int final_normalize, float* out, long long ld_out,
                       long long rows, int n_classes, const int* out_row_map, void* stream) {
   return nnam::head(logits_host, weights_host, n_inputs, ld_in, pre_normalize, rpl_w, rpl_b, rpl_lb, prior,
-                    prior_scale, final_normalize, out, ld_out, rows, n_classes, out_row_map, nullptr, 0, nullptr,
-                    static_cast<cudaStream_t>(stream));
+                    prior_scale, final_normalize, out, ld_out, rows, n_classes, out_row_map, nullptr, 0, nullptr, nullptr,
+                    nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int nnam_head_f16(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in,
@@ -159,8 +170,18 @@ int nnam_head_f16(const float* const* logits_host, const float* weights_host, in
                   int n_classes, const int* out_row_map, void* stream) {
   if (out16 == nullptr) return nnam::set_error(NNAM_ERR_ARG, "head_f16: out16 is NULL");
   return nnam::head(logits_host, weights_host, n_inputs, ld_in, pre_normalize, rpl_w, rpl_b, rpl_lb, prior,
-                    prior_scale, final_normalize, nullptr, 0, rows, n_classes, out_row_map, out16, ld16, row_ref,
-                    static_cast<cudaStream_t>(stream));
+                    prior_scale, final_normalize, nullptr, 0, rows, n_classes, out_row_map, out16, ld16, row_ref, nullptr,
+                    nullptr, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+int nnam_head_score(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in,
+                    int pre_normalize, const float* rpl_w, const float* rpl_b, const float* rpl_lb, const float* prior,
+                    float prior_scale, int final_normalize, const int* targets, float* nll, int* pred, long long rows,
+                    int n_classes, const int* out_row_map, void* stream) {
+  if (nll == nullptr) return nnam::set_error(NNAM_ERR_ARG, "head_score: nll is NULL");
+  return nnam::head(logits_host, weights_host, n_inputs, ld_in, pre_normalize, rpl_w, rpl_b, rpl_lb, prior,
+                    prior_scale, final_normalize, nullptr, 0, rows, n_classes, out_row_map, nullptr, 0, nullptr,
+                    targets, nll, pred, static_cast<cudaStream_t>(stream));
 }
 
 int nnam_gather_transform(const float* x, long long n_src, int dim, const float* add_shift, const float* rescale,

@@ -17,6 +17,12 @@
 //            a swizzled shared-memory box and leaves as 128-byte row segments (the (N, 1909) float32 rows are only
 //            4-byte aligned, so no TMA store), through the optional row map of the recurrent path
 //
+// A third instance scores the rows against targets instead of storing them (nnam_linear_logsoftmax_score): pass 2
+// computes the same values but stages and stores none; each thread keeps the (max, lowest column) of its half and the
+// value at the target column, the thread holding the target writes nll = -v_t, and a second st.async exchange -- on the
+// staging boxes, which this instance leaves unused, and a barrier of its own -- brings every half's (max, column) of a
+// row to cluster rank 0, which writes pred.  8 B per row leave the kernel instead of 4 * N.
+//
 // Accumulators are double-buffered in TMEM (2 x 256 columns), so the epilogue of block i -- including the exchange
 // latency -- overlaps the MMAs of block i+1.  Main loop as in gemm.cu's single-CTA kernel (TMA producer warp, one
 // elected MMA thread, SWIZZLE_128B operand ring).
@@ -43,6 +49,9 @@ constexpr int XCHG_BYTES = 2 * 2 * MAX_CLUSTER * BM * 8;  // [accumulator parity
 constexpr int ROWPTR_BYTES = 8 * 32 * 8;               // per epilogue warp: output address of each of its 32 rows
 constexpr int SMEM_BYTES = ST * (A_STAGE_BYTES + B_STAGE_BYTES) + 8 * BOX_BYTES + BN * 4 + XCHG_BYTES + ROWPTR_BYTES + 256;
 static_assert(SMEM_BYTES <= 227 * 1024, "fused output kernel: shared memory over budget");
+static_assert(XCHG_BYTES <= 8 * BOX_BYTES, "scoring instance: the argmax exchange lives in the staging boxes");
+// what pass 2 produces: float32 rows, the compact transfer format, or (nll, pred) against targets
+constexpr int OUT_ROWS = 0, OUT_COMPACT = 1, OUT_SCORE = 2;
 constexpr int TMEM_COLS = 512;
 constexpr float NEG_BIG = -3.0e38f;  // finite stand-in for -inf as the running maximum's start value
 constexpr float LOG2E = 1.4426950408889634f;
@@ -54,11 +63,22 @@ struct Params {
   const float* bias;
   const float* prior;
   float prior_scale;
-  float* out;  // float32 rows
+  // The scoring instance stores no rows: its outputs and targets (indexed by output row) share the row outputs' slots,
+  // which keeps the kernel parameters -- and the register allocation of the other two instances -- as they were.
+  union {
+    float* out;  // float32 rows
+    float* nll;
+  };
   long long ld_out;
-  uint16_t* out16;  // compact format (nnam_head_f16): fp16 offsets from the row maximum + row_ref
+  union {
+    uint16_t* out16;  // compact format (nnam_head_f16): fp16 offsets from the row maximum + row_ref
+    int* pred;
+  };
   long long ld16;
-  float* row_ref;
+  union {
+    float* row_ref;
+    const int* targets;
+  };
   const int* out_row_map;
 };
 
@@ -111,11 +131,13 @@ __device__ __forceinline__ void online_chunk(const uint32_t (&r)[32], const floa
   m = mn;
 }
 
-template <bool COMPACT>
+template <int MODE>
 __global__ void __maxnreg__(168)
     gemm_logsoftmax_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                            const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
                            const Params p) {
+  constexpr bool COMPACT = MODE == OUT_COMPACT;
+  constexpr bool SCORE = MODE == OUT_SCORE;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + ST * A_STAGE_BYTES;
@@ -128,7 +150,9 @@ __global__ void __maxnreg__(168)
   uint64_t* tfull_bar = empty_bar + ST;
   uint64_t* tempty_bar = tfull_bar + 2;
   uint64_t* x_bar = tempty_bar + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(x_bar + 2);
+  uint64_t* x2_bar = x_bar + 2;  // scoring instance: argmax exchange into rank 0
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(x2_bar + 2);
+  float2* xchg2 = reinterpret_cast<float2*>(smem_epi);  // [accumulator parity][source rank, half][row] (max, column)
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -157,6 +181,7 @@ __global__ void __maxnreg__(168)
       mbar_init(&tfull_bar[a], 1);
       mbar_init(&tempty_bar[a], 8);  // one arrive per epilogue warp
       mbar_init(&x_bar[a], 1);  // one arrive.expect_tx per block; the peers' st.async stores complete the bytes
+      if (SCORE) mbar_init(&x2_bar[a], 1);
     }
     fence_mbar_init();
   }
@@ -259,6 +284,7 @@ __global__ void __maxnreg__(168)
     int acc = 0;
     uint32_t acc_phase = 0;
     uint32_t x_phase = 0;  // bit a: phase of x_bar[a]
+    uint32_t x2_phase = 0;  // bit a: phase of x2_bar[a] (scoring instance, rank 0)
     for (int mb = cluster_id; mb < p.tiles_m; mb += n_clusters) {
       const long long grow = static_cast<long long>(mb) * BM + trow;
       long long orow = -1;
@@ -271,7 +297,7 @@ __global__ void __maxnreg__(168)
         }
       }
       // address of this row's first element of the warp's half, staged for the store loops (0: row not written)
-      {
+      if constexpr (!SCORE) {
         unsigned long long a = 0;
         if (orow >= 0)
           a = COMPACT ? reinterpret_cast<unsigned long long>(p.out16 + orow * p.ld16 + n0 + h0)
@@ -328,9 +354,42 @@ __global__ void __maxnreg__(168)
       const float sub = COMPACT ? mx : mx + log_sum;
       if (COMPACT && rank == 0 && hf == 0 && orow >= 0) p.row_ref[orow] = zero ? 0.0f : -log_sum;
 
+      // ---- pass 2 (scoring): the values the float32 instance stores, reduced to this half's (max, lowest column) and
+      // the value at the target column
+      float best = -CUDART_INF_F;
+      int bcol = valid > 0 ? n0 + h0 : 0x7fffffff;  // an all -inf half reports its first column
+      if constexpr (SCORE) {
+        const int t = (orow >= 0 && !zero) ? __ldg(p.targets + orow) : -1;
+        const int t_half = t - (n0 + h0);  // target column within this half; here only if in [0, valid)
+        float vt = 0.0f;
+        for (int c0 = 0; c0 < valid; c0 += 32) {
+          uint32_t r[32];
+          tmem_ld32(taddr + c0, r);
+          tmem_ld_wait();
+          const float4* b4 = reinterpret_cast<const float4*>(bias_h + c0);
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const float4 b = b4[j];
+            // columns >= N carry bias -inf: never above `best`
+            const float v[4] = {__uint_as_float(r[4 * j]) + (b.x - sub), __uint_as_float(r[4 * j + 1]) + (b.y - sub),
+                                __uint_as_float(r[4 * j + 2]) + (b.z - sub), __uint_as_float(r[4 * j + 3]) + (b.w - sub)};
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              if (v[e] > best) {
+                best = v[e];
+                bcol = n0 + h0 + c0 + 4 * j + e;
+              }
+              if (c0 + 4 * j + e == t_half) vt = v[e];
+            }
+          }
+        }
+        if (t_half >= 0 && t_half < valid) p.nll[orow] = -vt;
+        else if (rank == 0 && hf == 0 && orow >= 0 && t < 0) p.nll[orow] = 0.0f;  // ignore label or zero-fill row
+      }
+
       // ---- pass 2: second read of the accumulator, normalise, stage, store row segments
       constexpr int CH2 = COMPACT ? 64 : 32;  // columns per staged box (128 B per row)
-      for (int c0 = 0; c0 < valid; c0 += CH2) {
+      for (int c0 = 0; c0 < (SCORE ? 0 : valid); c0 += CH2) {
         uint4 chunks[8];
         {
           uint32_t r[CH2 / 32][32];
@@ -404,6 +463,30 @@ __global__ void __maxnreg__(168)
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty_bar[acc]);
+      if constexpr (SCORE) {
+        // every half's (max, column) of the row goes to rank 0, whose half-0 threads pick the lowest column among the
+        // maxima (sources in column order) and write pred
+        if (rank == 0 && warp == 4 && lane == 0) mbar_expect_tx(&x2_bar[acc], static_cast<uint32_t>(cl * 2 * BM * 8));
+        const uint32_t slot = smem_u32(xchg2 + (acc * 2 * MAX_CLUSTER + rank * 2 + hf) * BM + trow);
+        st_async_f32x2(mapa_shared(slot, 0u), best, __int_as_float(bcol), mapa_shared(smem_u32(&x2_bar[acc]), 0u));
+        if (rank == 0 && hf == 0) {
+          mbar_wait(&x2_bar[acc], (x2_phase >> acc) & 1u);
+          x2_phase ^= 1u << acc;
+          if (orow >= 0) {
+            float bv = -CUDART_INF_F;
+            int bc = 0x7fffffff;
+            for (int r = 0; r < 2 * cl; ++r) {
+              const float2 e = xchg2[(acc * 2 * MAX_CLUSTER + r) * BM + trow];
+              const int c = __float_as_int(e.y);
+              if (e.x > bv || (e.x == bv && c < bc)) {
+                bv = e.x;
+                bc = c;
+              }
+            }
+            p.pred[orow] = zero ? -1 : bc;
+          }
+        }
+      }
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1;
     }
@@ -420,9 +503,9 @@ __global__ void __maxnreg__(168)
   }
 }
 
-template <bool COMPACT>
+template <int MODE>
 static int launch(const CUtensorMap (&tm)[4], const Params& p, cudaStream_t stream) {
-  auto kernel = gemm_logsoftmax_kernel<COMPACT>;
+  auto kernel = gemm_logsoftmax_kernel<MODE>;
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
   if (e != cudaSuccess) return set_cuda_error(e, "linear_logsoftmax: cudaFuncSetAttribute");
   cudaLaunchConfig_t cfg = {};
@@ -453,8 +536,9 @@ static int launch(const CUtensorMap (&tm)[4], const Params& p, cudaStream_t stre
 
 int linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, const void* w_hi, const void* w_lo,
                       long long ldw, const float* bias, const float* prior, float prior_scale, float* out,
-                      long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map, int M,
-                      int N, int K, int nsplit, int elem, cudaStream_t stream) {
+                      long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map,
+                      const int* targets, float* nll, int* pred, int M, int N, int K, int nsplit, int elem,
+                      cudaStream_t stream) {
   using namespace fused;
   if (M <= 0 || N <= 0 || K <= 0) return set_error(NNAM_ERR_ARG, "linear_logsoftmax: empty problem");
   if (N > MAX_CLUSTER * BN)
@@ -471,8 +555,10 @@ int linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, const v
   if (lda < K || ldw < K) return set_error(NNAM_ERR_ARG, "linear_logsoftmax: leading dimension smaller than K");
   if ((need_a_lo && !a_lo) || (need_w_lo && !w_lo))
     return set_error(NNAM_ERR_ARG, "linear_logsoftmax: split passes need their lo operands");
-  if ((out == nullptr) == (out16 == nullptr))
-    return set_error(NNAM_ERR_ARG, "linear_logsoftmax: exactly one of out / out16 must be given");
+  if ((out != nullptr) + (out16 != nullptr) + (nll != nullptr) != 1)
+    return set_error(NNAM_ERR_ARG, "linear_logsoftmax: exactly one of out / out16 / nll must be given");
+  if (nll != nullptr && (targets == nullptr || pred == nullptr))
+    return set_error(NNAM_ERR_ARG, "linear_logsoftmax: scoring needs targets, nll and pred");
   if (out != nullptr && ld_out < N) return set_error(NNAM_ERR_ARG, "linear_logsoftmax: ld_out must be >= N");
   if (out16 != nullptr && (row_ref == nullptr || ld16 < N || ld16 % 8 || (reinterpret_cast<uintptr_t>(out16) & 15)))
     return set_error(NNAM_ERR_ARG, "linear_logsoftmax: compact output needs row_ref, ld16 >= N, ld16 %% 8 == 0, 16-byte alignment");
@@ -493,12 +579,18 @@ int linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, const v
   p.bias = bias;
   p.prior = prior;
   p.prior_scale = prior_scale;
-  p.out = out;
   p.ld_out = ld_out;
-  p.out16 = static_cast<uint16_t*>(out16);
   p.ld16 = ld16;
-  p.row_ref = row_ref;
   p.out_row_map = out_row_map;
+  if (nll != nullptr) {
+    p.nll = nll;
+    p.pred = pred;
+    p.targets = targets;
+  } else {
+    p.out = out;
+    p.out16 = static_cast<uint16_t*>(out16);
+    p.row_ref = row_ref;
+  }
 
   CUtensorMap tm[4];
   int rc;
@@ -508,7 +600,8 @@ int linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, const v
   tm[3] = tm[2];
   if (need_a_lo && (rc = encode_tmap_bf16_2d(&tm[1], a_lo, K, M, lda, BK, BM))) return rc;
   if (need_w_lo && (rc = encode_tmap_bf16_2d(&tm[3], w_lo, K, N, ldw, BK, BN))) return rc;
-  return out16 != nullptr ? launch<true>(tm, p, stream) : launch<false>(tm, p, stream);
+  if (nll != nullptr) return launch<OUT_SCORE>(tm, p, stream);
+  return out16 != nullptr ? launch<OUT_COMPACT>(tm, p, stream) : launch<OUT_ROWS>(tm, p, stream);
 }
 
 }  // namespace nnam

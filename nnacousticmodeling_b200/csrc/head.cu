@@ -42,6 +42,12 @@ struct HeadParams {
   uint16_t* out16;
   long long ld16;
   float* row_ref;
+  // scoring output (nnam_head_score): per output row q, nll[q] = -y[q][targets[q]] (0 when targets[q] < 0) and
+  // pred[q] = argmax_c y[q][c] (lowest column on ties); a zero-fill entry -2 - q gives nll[q] = 0, pred[q] = -1.
+  // `out` and `out16` are unused then: a row costs 8 B of output instead of 4 * C.
+  const int* targets;
+  float* nll;
+  int* pred;
 };
 
 __device__ __forceinline__ uint32_t head_pack_f16x2(float lo, float hi) { return pack_f16x2(lo, hi); }
@@ -55,6 +61,32 @@ __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// (value, column) of the row maximum, lowest column on ties, across the warp; every lane gets the result
+__device__ __forceinline__ void warp_argmax(float& best, int& col) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+    const int oc = __shfl_xor_sync(0xffffffffu, col, o);
+    if (ov > best || (ov == best && oc < col)) {
+      best = ov;
+      col = oc;
+    }
+  }
+}
+
+// Scoring epilogue of one row (one warp): `best` / `col` are this lane's running maximum over its columns (visited in
+// increasing order, strict > so the lowest column wins), `vt` the written value of column t if this lane holds it
+// (lane t_lane does).
+__device__ __forceinline__ void score_row(const HeadParams& p, long long q, bool zero, int t, int t_lane, float best,
+                                          int col, float vt, int lane) {
+  warp_argmax(best, col);
+  vt = __shfl_sync(0xffffffffu, vt, t_lane & 31);
+  if (lane == 0) {
+    p.nll[q] = (zero || t < 0) ? 0.0f : -vt;
+    p.pred[q] = zero ? -1 : col;
+  }
 }
 
 // log(sum(exp(v))) over the row held as v[i] <-> column lane + 32*i (invalid columns are skipped)
@@ -73,7 +105,7 @@ __device__ __forceinline__ float row_logsumexp(const float (&v)[NV], int lane, i
   return mx + logf(s);
 }
 
-template <int NV, bool MULTI>
+template <int NV, bool MULTI, bool SCORE>
 __global__ void __launch_bounds__(HEAD_THREADS, (MULTI || NV < 64) ? 1 : 2) head_kernel(const HeadParams p) {
   const int lane = threadIdx.x & 31;
   const long long warp_global = (static_cast<long long>(blockIdx.x) * HEAD_THREADS + threadIdx.x) >> 5;
@@ -138,6 +170,26 @@ __global__ void __launch_bounds__(HEAD_THREADS, (MULTI || NV < 64) ? 1 : 2) head
         zero = true;
       }
     }
+    if constexpr (SCORE) {
+      // the values the float32 path below writes, h[i] - lse
+      const int t = zero ? -1 : __ldg(p.targets + out_row);
+      float best = -CUDART_INF_F, vt = 0.0f;
+      int col = 0x7fffffff;
+#pragma unroll
+      for (int i = 0; i < NV; ++i) {
+        const int c = lane + 32 * i;
+        if (c < C) {
+          const float y = h[i] - lse;
+          if (y > best || col == 0x7fffffff) {
+            best = y;
+            col = c;
+          }
+          if (c == t) vt = y;
+        }
+      }
+      score_row(p, out_row, zero, t, t, best, col, vt, lane);
+      continue;
+    }
     if (p.out16 != nullptr) {
       float mx = -CUDART_INF_F;
 #pragma unroll
@@ -174,7 +226,7 @@ __global__ void __launch_bounds__(HEAD_THREADS, (MULTI || NV < 64) ? 1 : 2) head
 //     a = (row start / 4) mod 4) and store 16-byte aligned chunks; only the row's ragged ends are scalar stores.
 constexpr int HEAD_FAST_THREADS = 128;
 
-template <int NV4>
+template <int NV4, bool SCORE>
 __global__ void __launch_bounds__(HEAD_FAST_THREADS, 4) head_fast_kernel(const HeadParams p) {
   const int lane = threadIdx.x & 31;
   const long long warp_global = (static_cast<long long>(blockIdx.x) * HEAD_FAST_THREADS + threadIdx.x) >> 5;
@@ -250,16 +302,41 @@ __global__ void __launch_bounds__(HEAD_FAST_THREADS, 4) head_fast_kernel(const H
       lse = mx + logf(warp_sum(s0 + s1));
     }
     long long out_row = row;
+    bool zero = false;
     if (p.out_row_map != nullptr) {
       out_row = __ldg(p.out_row_map + row);
       if (out_row == -1) continue;  // warp-uniform: one row per warp
       if (out_row < 0) {            // -2 - r: fill output row r with zeros (quirk Q4 rows the reference never writes)
         out_row = -2 - out_row;
+        zero = true;
         lse = 0.0f;
         mx = 0.0f;
 #pragma unroll
         for (int i = 0; i < NV4; ++i) v[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
       }
+    }
+    if constexpr (SCORE) {
+      // the values the float32 path below writes, v - lse; a lane's columns 4k .. 4k+3 (k = lane + 32 i) increase with i
+      const int t = zero ? -1 : __ldg(p.targets + out_row);
+      float best = -CUDART_INF_F, vt = 0.0f;
+      int col = 0x7fffffff;
+#pragma unroll
+      for (int i = 0; i < NV4; ++i) {
+        const int c0 = 4 * (lane + 32 * i);
+        const float y[4] = {v[i].x - lse, v[i].y - lse, v[i].z - lse, v[i].w - lse};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          if (c0 + e < C) {
+            if (y[e] > best || col == 0x7fffffff) {
+              best = y[e];
+              col = c0 + e;
+            }
+            if (c0 + e == t) vt = y[e];
+          }
+        }
+      }
+      score_row(p, out_row, zero, t, t >> 2, best, col, vt, lane);  // column t sits in lane (t / 4) % 32
+      continue;
     }
     if (p.out16 != nullptr) {
       // rows of the fp16 matrix are 16-byte aligned (ld16 % 8 == 0): a lane's chunk k is one 8-byte store
@@ -312,16 +389,19 @@ __global__ void __launch_bounds__(HEAD_FAST_THREADS, 4) head_fast_kernel(const H
 int head(const float* const* logits_host, const float* weights_host, int n_inputs, long long ld_in, int pre_normalize,
          const float* rpl_w, const float* rpl_b, const float* rpl_lb, const float* prior, float prior_scale,
          int final_normalize, float* out, long long ld_out, long long rows, int n_classes, const int* out_row_map,
-         void* out16, long long ld16, float* row_ref, cudaStream_t stream) {
+         void* out16, long long ld16, float* row_ref, const int* targets, float* nll, int* pred, cudaStream_t stream) {
+  const bool score = nll != nullptr;
   if (n_inputs < 1 || n_inputs > HEAD_MAX_INPUTS)
     return set_error(NNAM_ERR_ARG, "head: n_inputs must be in [1, %d]", HEAD_MAX_INPUTS);
   if (n_classes < 1 || n_classes > 2048) return set_error(NNAM_ERR_UNSUPPORTED, "head: n_classes must be in [1, 2048]");
-  if (ld_in < n_classes || (out16 == nullptr && ld_out < n_classes))
+  if (ld_in < n_classes || (out16 == nullptr && !score && ld_out < n_classes))
     return set_error(NNAM_ERR_ARG, "head: leading dimension < n_classes");
   if (out16 != nullptr && (row_ref == nullptr || ld16 < n_classes || ld16 % 8 || (reinterpret_cast<uintptr_t>(out16) & 15)))
     return set_error(NNAM_ERR_ARG, "head: the fp16 output needs row_ref, ld16 >= n_classes, ld16 %% 8 == 0 and a "
                      "16-byte aligned buffer");
-  if (out16 == nullptr && out == nullptr) return set_error(NNAM_ERR_ARG, "head: no output buffer");
+  if (score && (targets == nullptr || pred == nullptr || out != nullptr || out16 != nullptr))
+    return set_error(NNAM_ERR_ARG, "head: scoring needs targets, nll and pred, and no row output");
+  if (out16 == nullptr && out == nullptr && !score) return set_error(NNAM_ERR_ARG, "head: no output buffer");
   if (rows < 0) return set_error(NNAM_ERR_ARG, "head: negative row count");
   if (rows == 0) return NNAM_OK;
   if ((rpl_w != nullptr) != (rpl_b != nullptr) || (rpl_w != nullptr) != (rpl_lb != nullptr))
@@ -349,6 +429,9 @@ int head(const float* const* logits_host, const float* weights_host, int n_input
   p.out16 = static_cast<uint16_t*>(out16);
   p.ld16 = ld16;
   p.row_ref = row_ref;
+  p.targets = targets;
+  p.nll = nll;
+  p.pred = pred;
   // fast path: one input, no RPL4 / per-input normalisation, 16-byte aligned input rows
   const bool fast_ok = n_inputs == 1 && !pre_normalize && rpl_w == nullptr && ld_in % 4 == 0 &&
                        (reinterpret_cast<uintptr_t>(logits_host[0]) & 15) == 0 &&
@@ -362,11 +445,19 @@ int head(const float* const* logits_host, const float* weights_host, int n_input
     if (fb > fcap) fb = fcap;
     const unsigned fg = static_cast<unsigned>(fb);
     const int need = n_classes + 3;  // see the kernel's closing comment
-    if (need <= 128) head_fast_kernel<1><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);
-    else if (need <= 512) head_fast_kernel<4><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);
-    else if (need <= 1024) head_fast_kernel<8><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);
-    else if (need <= 1920) head_fast_kernel<15><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);
-    else head_fast_kernel<16><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);
+#define NNAM_HEAD_FAST_LAUNCH(NV4)                                        \
+  do {                                                                    \
+    if (score)                                                            \
+      head_fast_kernel<NV4, true><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p);  \
+    else                                                                  \
+      head_fast_kernel<NV4, false><<<fg, HEAD_FAST_THREADS, 0, stream>>>(p); \
+  } while (0)
+    if (need <= 128) NNAM_HEAD_FAST_LAUNCH(1);
+    else if (need <= 512) NNAM_HEAD_FAST_LAUNCH(4);
+    else if (need <= 1024) NNAM_HEAD_FAST_LAUNCH(8);
+    else if (need <= 1920) NNAM_HEAD_FAST_LAUNCH(15);
+    else NNAM_HEAD_FAST_LAUNCH(16);
+#undef NNAM_HEAD_FAST_LAUNCH
     return check_launch("head_fast_kernel");
   }
   const int warps_per_block = HEAD_THREADS / 32;
@@ -377,10 +468,14 @@ int head(const float* const* logits_host, const float* weights_host, int n_input
   const unsigned g = static_cast<unsigned>(blocks);
 #define NNAM_HEAD_LAUNCH(NV)                                              \
   do {                                                                    \
-    if (multi)                                                            \
-      head_kernel<NV, true><<<g, HEAD_THREADS, 0, stream>>>(p);           \
+    if (score && multi)                                                   \
+      head_kernel<NV, true, true><<<g, HEAD_THREADS, 0, stream>>>(p);     \
+    else if (score)                                                       \
+      head_kernel<NV, false, true><<<g, HEAD_THREADS, 0, stream>>>(p);    \
+    else if (multi)                                                       \
+      head_kernel<NV, true, false><<<g, HEAD_THREADS, 0, stream>>>(p);    \
     else                                                                  \
-      head_kernel<NV, false><<<g, HEAD_THREADS, 0, stream>>>(p);          \
+      head_kernel<NV, false, false><<<g, HEAD_THREADS, 0, stream>>>(p);   \
   } while (0)
   if (n_classes <= 128)
     NNAM_HEAD_LAUNCH(4);

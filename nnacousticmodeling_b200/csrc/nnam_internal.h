@@ -25,7 +25,8 @@ int gemm_bias_act(const void* a_hi, const void* a_lo, long long lda, const void*
 
 int linear_logsoftmax(const void* a_hi, const void* a_lo, long long lda, const void* w_hi, const void* w_lo,
                       long long ldw, const float* bias, const float* prior, float prior_scale, float* out,
-                      long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map, int M,
-                      int N, int K, int nsplit, int elem, cudaStream_t stream);
+                      long long ld_out, void* out16, long long ld16, float* row_ref, const int* out_row_map,
+                      const int* targets, float* nll, int* pred, int M, int N, int K, int nsplit, int elem,
+                      cudaStream_t stream);
 
 }  // namespace nnam

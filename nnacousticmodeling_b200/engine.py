@@ -127,13 +127,14 @@ class LinearDev:
 
 
     def logsoftmax(self, a_hi, a_lo, rows, prior=None, prior_scale=1.0, nsplit=None, out=None, out16=None,
-                   out_row_map=None):
-        """This layer as the output layer of a single net, fused with the head (ops.linear_logsoftmax)."""
+                   out_row_map=None, score=None):
+        """This layer as the output layer of a single net, fused with the head (ops.linear_logsoftmax); ``score`` =
+        (targets, nll, pred) scores the rows instead of writing them."""
         if nsplit is None:
             nsplit = SPLIT_AW if self.split else SPLIT_NONE
         return ops.linear_logsoftmax(a_hi, a_lo, self.w_hi, self.w_lo, self.bias, rows, self.n, self.k, prior=prior,
                                      prior_scale=prior_scale, nsplit=nsplit, elem=self.elem, out=out, out16=out16,
-                                     out_row_map=out_row_map)
+                                     out_row_map=out_row_map, score=score)
 
 
 FUSED_HEAD_MAX_K = 1024
@@ -375,8 +376,30 @@ class RowSink:
         raise NotImplementedError
 
 
+def upload_targets(ws, name, targets, r0, r1):
+    """Rows [r0, r1) of the (N,) int32 host targets as a device vector in workspace memory (4 B per frame, once per
+    shard)."""
+    t = ws.get(name, r1 - r0, 1, torch.int32).view(-1)
+    t.copy_(torch.from_numpy(np.ascontiguousarray(targets[r0:r1], dtype=np.int32)))
+    return t
+
+
+def score_buffers(ws, tag, targets, r0, r1):
+    """Device (targets, nll, pred) of rows [r0, r1) for a scoring pass, in workspace memory (NNAM_REDZONE guards
+    them)."""
+    return (upload_targets(ws, f"{tag}.targets", targets, r0, r1), ws.get(f"{tag}.nll", r1 - r0, 1, torch.float32).view(-1),
+            ws.get(f"{tag}.pred", r1 - r0, 1, torch.int32).view(-1))
+
+
+def download_scores(dev, score, r0, r1):
+    """Copy the device (nll, pred) of rows [r0, r1) into the host arrays of ``score`` = (targets, nll, pred)."""
+    _, nll_h, pred_h = score
+    nll_h[r0:r1] = dev[1].cpu().numpy()
+    pred_h[r0:r1] = dev[2].cpu().numpy()
+
+
 def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, device=0, head=None,
-                      chunk=None, presliced=False, sink=None, transfer=None, host_threads=None):
+                      chunk=None, presliced=False, sink=None, transfer=None, host_threads=None, score=None):
     """Feed-forward hot loop on ONE device for frames [f0, f1) of the whole array ``x``.
 
     models    : one MLP or a list (ensemble -> logits combined in the head with head.weights)
@@ -392,6 +415,11 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                 nnam_head_f16 (fp16 offsets from the row maximum + the maximum: half the PCIe bytes, widened back to
                 float32 by ``host_threads`` host threads); None = "f16" in the 16-bit precision modes, "f32" in the
                 fp32-accurate mode (see :func:`use_compact_transfer`).
+    score     : (targets, nll, pred) host arrays of shape (N,) -- int32 targets in [-1, C), float32 nll, int32 pred --
+                to score rows [f0, f1) against their targets instead of writing them (``out`` and ``sink`` are None
+                then): nll[f] = -y[f][targets[f]] (0 for target -1), pred[f] = argmax_c y[f][c], with y the row this
+                function would have written to a host ``out``.  The targets go up once, the chunk sizes and kernel
+                choices are those of a host ``out``, and 8 B per frame come back at the end.
     """
     if not isinstance(models, (list, tuple)):
         models = [models]
@@ -462,7 +490,9 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         n_lin = len(getattr(plan0, "layers", ())) + 1
         out_on_device = isinstance(out, torch.Tensor) and out.is_cuda
         out_h = None if (out_on_device or out is None) else _as_host_tensor(out)
-        if out is None and sink is None:
+        if score is not None and (out is not None or sink is not None):
+            raise NnamError("ff_forward_frames: a scoring pass writes no rows (out and sink must be None)")
+        if out is None and sink is None and score is None:
             raise NnamError("ff_forward_frames: give an output array or a RowSink")
         chunk = min(chunk, f1 - f0)
         d_in = models[0].in_size
@@ -476,7 +506,9 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
             raise NnamError("ensemble members must use the same precision mode")
         a_bufs = [(ws.get("ff.a.hi", chunk, ld_in, plan0.tdt),
                    ws.get("ff.a.lo", chunk, ld_in, torch.bfloat16) if plan0.in_kind == OUT_BF16_SPLIT else None)]
-        out_dev = None if out_on_device else [ws.get(f"ff.out{i}", chunk, n_out, torch.float32) for i in range(2)]
+        out_dev = None if (out_on_device or score is not None) else [ws.get(f"ff.out{i}", chunk, n_out, torch.float32)
+                                                                      for i in range(2)]
+        sc_dev = None if score is None else score_buffers(ws, "ff", score[0], f0, f1)
         # Host output.  "direct" = D2H straight into the caller's array; otherwise a chunk goes through one of two pinned
         # staging buffers and a helper thread finishes it (widen the compact format and / or feed the sink).  With the
         # compact format and a PINNED destination the chunks are MIXED: PCIe and the widening threads are two servers,
@@ -484,7 +516,8 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         # chunks goes compact such that both finish together (see _TransferStats).
         host_threads = host_threads or default_host_threads()
         mixable = (not out_on_device) and sink is None and out_h is not None and out_h.is_pinned()
-        compact = (not out_on_device) and use_compact_transfer(plan0, transfer, host_threads=host_threads, mixable=mixable)
+        compact = (not out_on_device and score is None) and use_compact_transfer(plan0, transfer, host_threads=host_threads,
+                                                                                  mixable=mixable)
         writer = o16_dev = ref_dev = stats = None
         frac_compact = 1.0
         if (compact or sink is not None) and not out_on_device:
@@ -594,6 +627,8 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                 okw = dict(prior=prior, prior_scale=head.prior_scale, nsplit=plan0.prec.nsplit(n_lin - 1, n_lin))
                 if out_on_device:
                     plan0.out.logsoftmax(h_hi, h_lo, rows, out=out[c0:c1], **okw)
+                elif sc_dev is not None:
+                    plan0.out.logsoftmax(h_hi, h_lo, rows, score=tuple(t[c0 - f0:c1 - f0] for t in sc_dev), **okw)
                 else:
                     if last[ob] is not None:
                         main.wait_event(last[ob])  # the side stream still reads this buffer
@@ -615,6 +650,8 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                 with torch.cuda.stream(aux):
                     if out_on_device:
                         ops.head(logits, n_out, out=out[c0:c1], **hkw)
+                    elif sc_dev is not None:
+                        ops.head_score(logits, n_out, *(t[c0 - f0:c1 - f0] for t in sc_dev), **hkw)
                     else:
                         if last[ob] is not None:
                             aux.wait_event(last[ob])  # the side stream still reads this buffer
@@ -625,7 +662,7 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                     hd = torch.cuda.Event()
                     hd.record(aux)
             head_done[buf] = hd
-            if out_on_device:
+            if out_on_device or sc_dev is not None:
                 continue
             # the copies of chunk i are queued one iteration later, after chunk i+1's kernels: queueing them may block on
             # the helper thread (ring slots), and the GPU should have its next chunk by then
@@ -635,6 +672,8 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         if pending is not None:
             drain(*pending)
         main.wait_stream(aux)  # callers that time or consume on the current stream see the whole pass
+        if sc_dev is not None:
+            download_scores(sc_dev, score, f0, f1)
         side.synchronize()
         main.synchronize()
         if writer is not None:

@@ -154,11 +154,23 @@ def linear_bias_act(a_hi, a_lo, w_hi, w_lo, bias, M, N, K, act="identity", out_k
 FUSED_HEAD_MAX_CLASSES = 2048  # eight 256-column tiles: one thread-block cluster spans a row
 
 
+def _req_score(score):
+    targets, nll, pred = score
+    _req(targets, torch.int32, "targets")
+    _req(nll, torch.float32, "nll")
+    _req(pred, torch.int32, "pred")
+    if targets is None or nll is None or pred is None:
+        raise NnamError("scoring needs targets, nll and pred tensors")
+    return targets, nll, pred
+
+
 def linear_logsoftmax(a_hi, a_lo, w_hi, w_lo, bias, M, N, K, prior=None, prior_scale=1.0, nsplit=1, elem=ELEM_BF16,
-                      out=None, out16=None, out_row_map=None):
+                      out=None, out16=None, out_row_map=None, score=None):
     """K2 + K4 fused for one net without RPL: log_softmax(A . W^T + bias - prior_scale * prior) straight from the
     accumulators (the float32 logits never go to HBM).  ``out``: float32 (rows_out, >= N) tensor, or ``out16`` = (fp16
-    (rows_out, ld16), f32 (rows_out,)) for the compact transfer format; ``out_row_map`` as in :func:`head`."""
+    (rows_out, ld16), f32 (rows_out,)) for the compact transfer format; ``out_row_map`` as in :func:`head`.
+    ``score`` = (int32 targets, f32 nll, int32 pred), each indexed by output row, scores the rows the float32 form would
+    write instead of writing them (nnam_linear_logsoftmax_score); returns that tuple."""
     for t, n in ((a_hi, "a_hi"), (w_hi, "w_hi")):
         _req(t, E16[elem], n)
     for t, n in ((a_lo, "a_lo"), (w_lo, "w_lo")):
@@ -170,6 +182,14 @@ def linear_logsoftmax(a_hi, a_lo, w_hi, w_lo, bias, M, N, K, prior=None, prior_s
         a_lo = None
     if nsplit in (SPLIT_NONE, SPLIT_A):
         w_lo = None
+    if score is not None:
+        targets, nll, pred = _req_score(score)
+        with _Prof("gemm", 2.0 * M * N * K):
+            check(_native.lib().nnam_linear_logsoftmax_score(
+                _ptr(a_hi), _ptr(a_lo), a_hi.stride(0), _ptr(w_hi), _ptr(w_lo), w_hi.stride(0), _ptr(bias), _ptr(prior),
+                float(prior_scale), _ptr(targets), _ptr(nll), _ptr(pred), _ptr(out_row_map), M, N, K, nsplit, elem,
+                _stream()))
+        return score
     o16 = ref = None
     if out16 is not None:
         o16, ref = out16
@@ -237,6 +257,38 @@ def head(logits, n_classes, rows=None, weights=None, pre_normalize=False, rpl=No
                                                   int(bool(final_normalize)), _ptr(out), out.stride(0), rows,
                                                   n_classes, _ptr(out_row_map), _stream()))
     return out
+
+
+def head_score(logits, n_classes, targets, nll, pred, rows=None, weights=None, pre_normalize=False, rpl=None, prior=None,
+               prior_scale=1.0, final_normalize=True, out_row_map=None):
+    """K4 scored against frame targets (nnam_head_score): the rows :func:`head` would write are reduced to nll[q] =
+    -y[q][targets[q]] (0 for target -1) and pred[q] = argmax_c y[q][c] (lowest column on ties); a zero-fill map entry
+    -2 - q gives nll 0, pred -1.  ``targets`` / ``nll`` / ``pred``: int32 / f32 / int32, indexed by output row."""
+    if isinstance(logits, torch.Tensor):
+        logits = [logits]
+    for t in logits:
+        _req(t, torch.float32, "logits")
+    ld_in = logits[0].stride(0)
+    if any(t.stride(0) != ld_in for t in logits):
+        raise NnamError("head: all inputs must share one leading dimension")
+    if rows is None:
+        rows = logits[0].shape[0]
+    targets, nll, pred = _req_score((targets, nll, pred))
+    k = len(logits)
+    ptrs = (ctypes.c_void_p * k)(*[t.data_ptr() for t in logits])
+    wts = None if weights is None else (ctypes.c_float * k)(*[float(w) for w in weights])
+    rw = rb = rlb = None
+    if rpl is not None:
+        rw, rb, rlb = rpl
+        for t in (rw, rb, rlb):
+            _req(t, torch.float32, "rpl")
+    _req(prior, torch.float32, "prior")
+    _req(out_row_map, torch.int32, "out_row_map")
+    with _Prof("head", rows * (n_classes * 4 * k + 12)):
+        check(_native.lib().nnam_head_score(ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb), _ptr(rlb),
+                                            _ptr(prior), float(prior_scale), int(bool(final_normalize)), _ptr(targets),
+                                            _ptr(nll), _ptr(pred), rows, n_classes, _ptr(out_row_map), _stream()))
+    return nll, pred
 
 
 def widen_f16_host(src16, row_ref, dst, threads=1, dst_rows=None):

@@ -113,9 +113,10 @@ def _activation(name):
     return F.resolve(name)
 
 
-def main(arg_list=None):
-    """predict_folds.py:97-246 -- same flags, same directory conventions, same outputs."""
-    parser = argparse.ArgumentParser(description="B200 network-output step (predict_folds drop-in)")
+def fold_arg_parser(description):
+    """The predict_folds flags (predict_folds.py:97-130) with their names and defaults, shared by this module's CLI and
+    the scoring CLI (score.main)."""
+    parser = argparse.ArgumentParser(description=description)
     parser.add_argument("--network", "-n", default="ff")
     parser.add_argument("--gpu", "-g", type=int, nargs="+", default=[0], help="GPU id(s); CPU (<0) is not supported")
     parser.add_argument("--units", "-u", type=int, nargs="+", default=[1024])
@@ -144,10 +145,11 @@ def main(arg_list=None):
     parser.add_argument("--fold-network-pattern", default="fold_{}.npz")
     parser.add_argument("--no-progress", action="store_true")
     parser.add_argument("--precision", default=None, help="extension: GEMM precision mode (fp32 | fp16 | bf16, see engine.Precision)")
-    args = parser.parse_args(list(map(str, arg_list)) if arg_list is not None else None)
+    return parser
 
-    out_file = Path(args.fold_output_dir, args.fold_output_dev or args.fold_output_pattern)
-    out_file.parent.mkdir(exist_ok=True, parents=True)
+
+def fold_setup(args):
+    """What both fold CLIs derive from the flags: (model, its Classifier, num_classes, recurrent, winlen, ft, gpu)."""
     num_classes = 1909 if args.tri else 39
     model = get_nn(args.network, args.layers, args.units, num_classes, _activation(args.activation),
                    args.tdnn_ksize, args.dropout)
@@ -162,6 +164,17 @@ def main(arg_list=None):
         ft = adapt_transform(loadKaldiFeatureTransform(str(Path(args.data_dir, args.ft))), args.network, splice,
                              recurrent)
     gpu = args.gpu if len(args.gpu) > 1 else args.gpu[0]
+    return model, model_cls, num_classes, recurrent, winlen, ft, gpu
+
+
+def main(arg_list=None):
+    """predict_folds.py:97-246 -- same flags, same directory conventions, same outputs."""
+    parser = fold_arg_parser("B200 network-output step (predict_folds drop-in)")
+    args = parser.parse_args(list(map(str, arg_list)) if arg_list is not None else None)
+
+    out_file = Path(args.fold_output_dir, args.fold_output_dev or args.fold_output_pattern)
+    out_file.parent.mkdir(exist_ok=True, parents=True)
+    model, model_cls, num_classes, recurrent, winlen, ft, gpu = fold_setup(args)
 
     def fold_models():
         fold = 0

@@ -717,10 +717,11 @@ def _phase_split(lens):
 
 
 def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, out_dev, timedelay, fix_timedelay_tail,
-                   nb, device, stepwise, out16=None, out_starts=None):
+                   nb, device, stepwise, out16=None, out_starts=None, score=None):
     """One subset of utterances (start frame relative to the shard and length of each) through the whole net:
     packed gather -> layers -> output GEMM -> head, which scatters the rows into ``out_dev`` (all frames of the shard)
-    or, with ``out16`` = (fp16 rows, row maxima), into the compact transfer format (ops.head).  ``out_starts``: first
+    or, with ``out16`` = (fp16 rows, row maxima), into the compact transfer format (ops.head), or, with ``score`` =
+    device (targets, nll, pred) of all frames of the shard, scores them (ops.head_score).  ``out_starts``: first
     OUTPUT row of every utterance when that differs from its first input frame (the compact format packs the rows of a
     subset one after the other)."""
     if out_starts is None:
@@ -791,17 +792,29 @@ def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, o
         pl.out(h_hi, h_lo, rows, "identity", OUT_F32, out=(lg, None))
         logits.append(lg)
     for u in np.nonzero(lens < timedelay)[0]:  # utterances shorter than the delay have rows no packed row maps to
+        r0, r1 = int(out_starts[u]), int(out_starts[u] + lens[u])
+        if score is not None:
+            score[1][r0:r1].zero_()
+            score[2][r0:r1].fill_(-1)
+            continue
         for t in ((out_dev,) if out16 is None else out16):
-            t[int(out_starts[u]):int(out_starts[u] + lens[u])].zero_()
+            t[r0:r1].zero_()
     prior = _dev_vec(head.prior, device)
     rpl = None if head.rpl is None else tuple(_dev_vec(head.rpl[k], device) for k in ("W", "b", "lb"))
     if fused:
+        if score is not None:
+            plans[0].out.logsoftmax(h_hi, h_lo, rows, prior=prior, prior_scale=head.prior_scale, out_row_map=d_dst,
+                                    score=score)
+            return
         plans[0].out.logsoftmax(h_hi, h_lo, rows, prior=prior, prior_scale=head.prior_scale, out_row_map=d_dst,
                                 out=None if out16 is not None else out_dev, out16=out16)
         return
-    ops.head(logits, n_out, rows=rows, weights=head.weights, pre_normalize=head.pre_normalize, rpl=rpl, prior=prior,
-             prior_scale=head.prior_scale, final_normalize=head.final_normalize, out=out_dev, out_row_map=d_dst,
-             out16=out16)
+    hkw = dict(rows=rows, weights=head.weights, pre_normalize=head.pre_normalize, rpl=rpl, prior=prior,
+               prior_scale=head.prior_scale, final_normalize=head.final_normalize, out_row_map=d_dst)
+    if score is not None:
+        ops.head_score(logits, n_out, *score, **hkw)
+        return
+    ops.head(logits, n_out, out=out_dev, out16=out16, **hkw)
 
 
 class _PackedDrainer:
@@ -883,7 +896,7 @@ class _PackedDrainer:
 
 
 def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, timedelay=0, device=0, head=None,
-                       fix_timedelay_tail=False, nb=DEFAULT_BATCH, transfer=None, host_threads=None):
+                       fix_timedelay_tail=False, nb=DEFAULT_BATCH, transfer=None, host_threads=None, score=None):
     """Recurrent hot path on ONE device for utterances [u0, u1) (predict_folds.py:28-68 semantics).
 
     model: one recurrent spec or a list of them (ensemble: the logits are combined in the head, evaluate.py:35-51).
@@ -894,6 +907,10 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
     the first one to the host runs under the computation of the second.  ``transfer`` / ``host_threads``: as in
     engine.ff_forward_frames -- in the 16-bit modes the rows cross PCIe in the compact format (fp16 offsets from the row
     maximum) into a pinned staging area and host threads widen them into ``out`` while the GPU computes the next subset.
+    ``score``: (targets, nll, pred) host arrays of shape (N,) to score the rows against their targets instead of writing
+    them (``out`` is None then), as in engine.ff_forward_frames.  The targets go up once per shard in frame order (the
+    kernels index them by output row, so the packed order needs no gather); the utterance subsets, schedules and kernel
+    choices are those of a host ``out``, and 8 B per frame come back at the end of the shard.
     """
     models = list(model) if isinstance(model, (list, tuple)) else [model]
     device = _device(device)
@@ -938,9 +955,15 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
         n_out = models[0].n_out
         on_dev = isinstance(out, torch.Tensor) and out.is_cuda
         n_rows = f_hi - f_lo
-        compact = (not on_dev) and engine.use_compact_transfer(plan, transfer, recurrent=True, host_threads=host_threads)
-        out16 = None
-        if compact:
+        if score is not None and out is not None:
+            raise NnamError("forward_utterances: a scoring pass writes no rows (out must be None)")
+        compact = (not on_dev and score is None) and engine.use_compact_transfer(plan, transfer, recurrent=True,
+                                                                                 host_threads=host_threads)
+        out16 = sc_dev = None
+        if score is not None:
+            sc_dev = engine.score_buffers(ws, "rnn", score[0], f_lo, f_hi)
+            out_dev = None
+        elif compact:
             ld16 = round_up(n_out, 8)
             out16 = (ws.get("rnn.out16", n_rows, ld16, torch.float16), ws.get("rnn.ref", n_rows, 1, torch.float32).view(-1))
             out_dev = None
@@ -961,8 +984,8 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
                 if compact:
                     o_starts = packed + np.concatenate([[0], np.cumsum(p_lens[:-1])]).astype(np.int64)
                 _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, p_starts, p_lens, out_dev, timedelay,
-                               fix_timedelay_tail, nb, device, stepwise, out16=out16, out_starts=o_starts)
-                if on_dev:
+                               fix_timedelay_tail, nb, device, stepwise, out16=out16, out_starts=o_starts, score=sc_dev)
+                if on_dev or sc_dev is not None:
                     continue
                 out_host = None if compact else _as_host_tensor(out)
                 if len(phases) == 1 and not compact:
@@ -996,6 +1019,8 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
         finally:
             if drainer is not None:  # an error above: let the helper thread go
                 drainer.abort()
+        if sc_dev is not None:
+            engine.download_scores(sc_dev, score, f_lo, f_hi)
         main.synchronize()
         if side is not None:
             side.synchronize()
