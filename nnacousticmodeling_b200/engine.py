@@ -361,6 +361,62 @@ class HeadSpec:
         self.prior, self.prior_scale, self.rpl = prior, prior_scale, rpl
         self.weights, self.pre_normalize, self.final_normalize = weights, pre_normalize, final_normalize
 
+    def device_args(self, device):
+        """The keyword arguments of ops.head, with the prior and RPL vectors uploaded to ``device``."""
+        rpl = None if self.rpl is None else tuple(_dev_vec(self.rpl[k], device) for k in ("W", "b", "lb"))
+        return dict(prior=_dev_vec(self.prior, device), prior_scale=self.prior_scale, rpl=rpl, weights=self.weights,
+                    pre_normalize=self.pre_normalize, final_normalize=self.final_normalize)
+
+
+def run_head(hargs, dest, rows, out_row_map=None, logits=None, n_out=None, fused=None, h=None, nsplit=None):
+    """The head over ``rows`` rows on the current stream: from the ``logits`` of the ensemble members (ops.head,
+    ``hargs`` = HeadSpec.device_args), or, with ``fused`` = the output layer (see fused_head_ok), that layer and the head
+    as one kernel on its operands ``h`` = (hi, lo).  ``dest``, the head's DESTINATION, is the one keyword of those ops
+    that says where the rows go, sliced to the rows being produced: {"out": float32 rows}, {"out16": (fp16 rows, row
+    maxima)} (the compact transfer format) or {"score": (targets, nll, pred)} (the rows scored against their targets
+    instead of written)."""
+    if fused is not None:
+        return fused.logsoftmax(h[0], h[1], rows, prior=hargs["prior"], prior_scale=hargs["prior_scale"], nsplit=nsplit,
+                                out_row_map=out_row_map, **dest)
+    return ops.head(logits, n_out, rows=rows, out_row_map=out_row_map, **hargs, **dest)
+
+
+def zero_rows(dest, r0, r1):
+    """Rows [r0, r1) of ``dest`` as the head leaves a row its row map zero-fills: 0 (in both planes of the compact
+    format), or nll 0 and pred -1 when scoring."""
+    (kind, val), = dest.items()
+    if kind == "score":
+        val[1][r0:r1].zero_()
+        val[2][r0:r1].fill_(-1)
+    else:
+        for t in ((val,) if kind == "out" else val):
+            t[r0:r1].zero_()
+
+
+def check_ensemble(models, plans, who=""):
+    """Ensemble members are combined row by row in one head: they must agree on sizes and precision mode."""
+    if any(m.in_size != models[0].in_size or m.n_out != models[0].n_out for m in models):
+        raise NnamError(f"{who}ensemble members must share input and output sizes")
+    if any(p.prec.spec != plans[0].prec.spec for p in plans):
+        raise NnamError(f"{who}ensemble members must use the same precision mode")
+
+
+def staging_ring(plan, compact, rows, n_out):
+    """Pinned host buffers that host-bound output rows cross PCIe into, kept on ``plan`` for the next pass (a pass of
+    another shape replaces them): NNAM_PIECE_SLOTS pieces of ``rows`` rows of the compact format (fp16 rows, row
+    maxima), or two chunks of ``rows`` float32 rows."""
+    slots = max(2, int(os.environ.get("NNAM_PIECE_SLOTS", "4")))
+    key = ("f16" if compact else "f32", rows, n_out, slots)
+    cache = plan.__dict__.setdefault("_stage", {})
+    if key not in cache:
+        cache.clear()
+        if compact:
+            cache[key] = [(torch.empty((rows, round_up(n_out, 8)), dtype=torch.float16, pin_memory=True),
+                           torch.empty((rows,), dtype=torch.float32, pin_memory=True)) for _ in range(slots)]
+        else:
+            cache[key] = [(torch.empty((rows, n_out), dtype=torch.float32, pin_memory=True), None) for _ in range(2)]
+    return cache[key]
+
 
 def _dev_vec(a, device):
     return None if a is None else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32).reshape(-1)).to(device)
@@ -434,6 +490,7 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
     lo, hi = halo_range(f0, f1, 0 if presliced else splice, n_total)
     with torch.cuda.device(device):
         plans = [get_plan(m, device) for m in models]
+        check_ensemble(models, plans)
         plan0 = plans[0]
         ws = plan0.ws
         t_pass = time.perf_counter()
@@ -484,8 +541,7 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         add = mul = None
         if ft is not None and not presliced:
             add, mul = _dev_vec(ft["addShift"], device), _dev_vec(ft["rescale"], device)
-        prior = _dev_vec(head.prior, device)
-        rpl = None if head.rpl is None else tuple(_dev_vec(head.rpl[k], device) for k in ("W", "b", "lb"))
+        hargs = head.device_args(device)
         fused = fused_head_ok(models, head, plan0.out.k if hasattr(plan0, "out") else 0)
         n_lin = len(getattr(plan0, "layers", ())) + 1
         out_on_device = isinstance(out, torch.Tensor) and out.is_cuda
@@ -496,14 +552,10 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
             raise NnamError("ff_forward_frames: give an output array or a RowSink")
         chunk = min(chunk, f1 - f0)
         d_in = models[0].in_size
-        if any(m.in_size != d_in or m.n_out != n_out for m in models):
-            raise NnamError("ensemble members must share input and output sizes")
         have = x.shape[1] if presliced else (2 * splice + 1) * x.shape[1] + (0 if ivectors is None else ivectors.shape[1])
         if have != d_in:
             raise NnamError(f"model expects {d_in} inputs per frame, the data provides {have}")
         ld_in = round_up(d_in, 8)
-        if any(p.prec.spec != plan0.prec.spec for p in plans):
-            raise NnamError("ensemble members must use the same precision mode")
         a_bufs = [(ws.get("ff.a.hi", chunk, ld_in, plan0.tdt),
                    ws.get("ff.a.lo", chunk, ld_in, torch.bfloat16) if plan0.in_kind == OUT_BF16_SPLIT else None)]
         out_dev = None if (out_on_device or score is not None) else [ws.get(f"ff.out{i}", chunk, n_out, torch.float32)
@@ -521,25 +573,14 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         writer = o16_dev = ref_dev = stats = None
         frac_compact = 1.0
         if (compact or sink is not None) and not out_on_device:
-            ld16 = round_up(n_out, 8)
             # Compact chunks cross PCIe in PIECES of a few thousand rows through a small ring of pinned buffers (4 x 16 MB
             # for 1909 classes): the widening threads then read a piece while it is still in the last-level cache (the
             # DMA wrote it there or it was just brought in), instead of streaming a 250 MB chunk back from DRAM -- the
             # widening is bound by the host's memory system, and this takes a third of its traffic away.
             piece = max(256, min(chunk, int(os.environ.get("NNAM_PIECE_ROWS", "4096")))) if compact else chunk
-            slots = max(2, int(os.environ.get("NNAM_PIECE_SLOTS", "4")))
-            key = ("f16" if compact else "f32", piece, n_out, slots)
-            cache = plan0.__dict__.setdefault("_stage", {})
-            if key not in cache:
-                cache.clear()
-                if compact:
-                    cache[key] = [(torch.empty((piece, ld16), dtype=torch.float16, pin_memory=True),
-                                   torch.empty((piece,), dtype=torch.float32, pin_memory=True)) for _ in range(slots)]
-                else:
-                    cache[key] = [(torch.empty((chunk, n_out), dtype=torch.float32, pin_memory=True), None) for _ in range(2)]
-            stage = cache[key]
+            stage = staging_ring(plan0, compact, piece, n_out)
             if compact:
-                o16_dev = [ws.get(f"ff.out16.{i}", chunk, ld16, torch.float16) for i in range(2)]
+                o16_dev = [ws.get(f"ff.out16.{i}", chunk, round_up(n_out, 8), torch.float16) for i in range(2)]
                 ref_dev = [ws.get(f"ff.ref.{i}", chunk, 1, torch.float32).view(-1) for i in range(2)]
                 if mixable and (transfer or os.environ.get("NNAM_TRANSFER")) is None:
                     stats = plan0.__dict__.setdefault("_xfer_stats", _TransferStats(host_threads))
@@ -559,31 +600,14 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
         copies = []                # (start, end, bytes) of every D2H copy, for the transfer statistics
         head_done = [None, None]   # head of the chunk that last used the logits buffers of this parity
         pending = None
-        ring = [0]
 
         def drain(as_compact, via_writer, ob, c0, c1, hd):
             """Queue the device->host copies of a finished chunk (rows [c0, c1)) and hand them to the helper thread."""
             rows = c1 - c0
             side.wait_event(hd)
-            ev = None
             if as_compact:
-                for p0 in range(0, rows, piece):
-                    p1 = min(p0 + piece, rows)
-                    slot = ring[0] % len(stage)
-                    ring[0] += 1
-                    writer.wait_free(slot)  # the helper thread still widens the piece that used this slot
-                    with torch.cuda.stream(side):
-                        t0 = torch.cuda.Event(enable_timing=True) if stats is not None else None
-                        if t0 is not None:
-                            t0.record(side)
-                        stage[slot][0][:p1 - p0].copy_(o16_dev[ob][p0:p1], non_blocking=True)
-                        stage[slot][1][:p1 - p0].copy_(ref_dev[ob][p0:p1], non_blocking=True)
-                        ev = torch.cuda.Event(enable_timing=stats is not None)
-                        ev.record(side)
-                        if stats is not None:
-                            copies.append((t0, ev, (p1 - p0) * (o16_dev[ob].stride(0) * 2 + 4)))
-                    writer.submit(slot, c0 + p0, c0 + p1, ev)
-                copied_c[ob] = ev
+                copied_c[ob] = writer.ship(side, (o16_dev[ob], ref_dev[ob]), rows, c0,
+                                           copies if stats is not None else None)
                 return
             if via_writer:
                 writer.wait_free(ob)  # the helper thread still reads the staging buffer of the chunk two before
@@ -620,22 +644,19 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                 ob, n_c = n_c % 2, n_c + 1   # ring position among the compact chunks / the staging buffers
             else:
                 ob, n_f = n_f % 2, n_f + 1   # ring position among the float32 chunks
-            last = copied_c if as_compact else copied_f
+            if out_on_device:
+                dest = {"out": out[c0:c1]}
+            elif sc_dev is not None:
+                dest = {"score": tuple(t[c0 - f0:c1 - f0] for t in sc_dev)}
+            else:
+                dest = {"out16": (o16_dev[ob], ref_dev[ob])} if as_compact else {"out": out_dev[ob]}
+            last = (copied_c if as_compact else copied_f)[ob]  # D2H still reading a staged destination (else None)
             if fused:
                 # output layer + head as ONE kernel on the main stream (no logits buffer, nothing for `aux` to do)
-                h_hi, h_lo = mlp_hidden(models[0], plan0, a_hi, a_lo, rows, ws)
-                okw = dict(prior=prior, prior_scale=head.prior_scale, nsplit=plan0.prec.nsplit(n_lin - 1, n_lin))
-                if out_on_device:
-                    plan0.out.logsoftmax(h_hi, h_lo, rows, out=out[c0:c1], **okw)
-                elif sc_dev is not None:
-                    plan0.out.logsoftmax(h_hi, h_lo, rows, score=tuple(t[c0 - f0:c1 - f0] for t in sc_dev), **okw)
-                else:
-                    if last[ob] is not None:
-                        main.wait_event(last[ob])  # the side stream still reads this buffer
-                    if as_compact:
-                        plan0.out.logsoftmax(h_hi, h_lo, rows, out16=(o16_dev[ob], ref_dev[ob]), **okw)
-                    else:
-                        plan0.out.logsoftmax(h_hi, h_lo, rows, out=out_dev[ob], **okw)
+                h = mlp_hidden(models[0], plan0, a_hi, a_lo, rows, ws)
+                if last is not None:
+                    main.wait_event(last)
+                run_head(hargs, dest, rows, fused=plan0.out, h=h, nsplit=plan0.prec.nsplit(n_lin - 1, n_lin))
                 hd = torch.cuda.Event()
                 hd.record(main)
             else:
@@ -644,21 +665,11 @@ def ff_forward_frames(models, x, ft, splice, out, f0=0, f1=None, ivectors=None, 
                 logits = [ff_logits(m, p, a_hi, a_lo, rows, f"ff{k}.{buf}", ws) for k, (m, p) in enumerate(zip(models, plans))]
                 gemm_done = torch.cuda.Event()
                 gemm_done.record(main)
-                hkw = dict(rows=rows, weights=head.weights, pre_normalize=head.pre_normalize, rpl=rpl, prior=prior,
-                           prior_scale=head.prior_scale, final_normalize=head.final_normalize)
                 aux.wait_event(gemm_done)
                 with torch.cuda.stream(aux):
-                    if out_on_device:
-                        ops.head(logits, n_out, out=out[c0:c1], **hkw)
-                    elif sc_dev is not None:
-                        ops.head_score(logits, n_out, *(t[c0 - f0:c1 - f0] for t in sc_dev), **hkw)
-                    else:
-                        if last[ob] is not None:
-                            aux.wait_event(last[ob])  # the side stream still reads this buffer
-                        if as_compact:
-                            ops.head(logits, n_out, out16=(o16_dev[ob], ref_dev[ob]), **hkw)
-                        else:
-                            ops.head(logits, n_out, out=out_dev[ob], **hkw)
+                    if last is not None:
+                        aux.wait_event(last)
+                    run_head(hargs, dest, rows, logits=logits, n_out=n_out)
                     hd = torch.cuda.Event()
                     hd.record(aux)
             head_done[buf] = hd
@@ -794,6 +805,7 @@ class _ChunkWriter:
         self.scratch = None
         self.widen_s, self.widen_bytes = 0.0, 0
         self.free = [threading.Event() for _ in stage]
+        self.k = 0  # pieces shipped so far: the next one goes to slot k % len(stage)
         for e in self.free:
             e.set()
         self.q = queue.Queue()
@@ -849,6 +861,35 @@ class _ChunkWriter:
 
     def submit(self, buf, r0, r1, ev):
         self.q.put((buf, r0, r1, ev))
+
+    def ship(self, side, src, n, dst, copies=None):
+        """Copy the first ``n`` rows of the compact format ``src`` = (fp16 rows, row maxima) on the device through the
+        ring of pinned pieces on the copy stream ``side``, and finish each piece on the helper thread once it has landed.
+        ``dst``: the output row of the first source row (the rows are consecutive), or an int64 array holding the output
+        row of every source row.  ``copies``: collects (start, end, bytes) of every copy, as timed CUDA events, for
+        _TransferStats.  Returns the event after the last copy."""
+        piece = self.stage[0][0].shape[0]
+        ev = None
+        for p0 in range(0, n, piece):
+            p1 = min(p0 + piece, n)
+            slot = self.k % len(self.stage)
+            self.k += 1
+            self.wait_free(slot)  # the helper thread still widens the piece that used this slot
+            with torch.cuda.stream(side):
+                if copies is not None:
+                    t0 = torch.cuda.Event(enable_timing=True)
+                    t0.record(side)
+                self.stage[slot][0][:p1 - p0].copy_(src[0][p0:p1], non_blocking=True)
+                self.stage[slot][1][:p1 - p0].copy_(src[1][p0:p1], non_blocking=True)
+                ev = torch.cuda.Event(enable_timing=copies is not None)
+                ev.record(side)
+                if copies is not None:
+                    copies.append((t0, ev, (p1 - p0) * (src[0].stride(0) * 2 + 4)))
+            if isinstance(dst, np.ndarray):
+                self.submit(slot, 0, dst[p0:p1], ev)
+            else:
+                self.submit(slot, dst + p0, dst + p1, ev)
+        return ev
 
     def close(self):
         self.q.put(None)

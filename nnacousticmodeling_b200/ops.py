@@ -210,9 +210,12 @@ def linear_logsoftmax(a_hi, a_lo, w_hi, w_lo, bias, M, N, K, prior=None, prior_s
 
 
 def head(logits, n_classes, rows=None, weights=None, pre_normalize=False, rpl=None, prior=None, prior_scale=1.0,
-         final_normalize=True, out=None, out_row_map=None, out16=None):
+         final_normalize=True, out=None, out_row_map=None, out16=None, score=None):
     """K4.  logits: one (rows, ld) f32 tensor or a list of them (ensemble).  ``out16`` = (fp16 (rows_out, ld16), f32
-    (rows_out,)) selects the compact transfer format (nnam_head_f16) instead of the float32 ``out``."""
+    (rows_out,)) selects the compact transfer format (nnam_head_f16) instead of the float32 ``out``.  ``score`` =
+    (int32 targets, f32 nll, int32 pred), each indexed by output row, scores the rows the float32 form would write
+    instead of writing them (nnam_head_score): nll[q] = -y[q][targets[q]] (0 for target -1) and pred[q] = argmax_c
+    y[q][c] (lowest column on ties); a zero-fill map entry -2 - q gives nll 0, pred -1.  Returns that tuple."""
     if isinstance(logits, torch.Tensor):
         logits = [logits]
     for t in logits:
@@ -222,7 +225,9 @@ def head(logits, n_classes, rows=None, weights=None, pre_normalize=False, rpl=No
         raise NnamError("head: all inputs must share one leading dimension")
     if rows is None:
         rows = logits[0].shape[0]
-    if out16 is not None:
+    if score is not None:
+        targets, nll, pred = _req_score(score)
+    elif out16 is not None:
         o16, ref = out16
         _req(o16, torch.float16, "out16")
         _req(ref, torch.float32, "row_ref")
@@ -239,56 +244,25 @@ def head(logits, n_classes, rows=None, weights=None, pre_normalize=False, rpl=No
             _req(t, torch.float32, "rpl")
     _req(prior, torch.float32, "prior")
     _req(out_row_map, torch.int32, "out_row_map")
+    args = (ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb), _ptr(rlb), _ptr(prior), float(prior_scale),
+            int(bool(final_normalize)))
+    if score is not None:
+        with _Prof("head", rows * (n_classes * 4 * k + 12)):
+            check(_native.lib().nnam_head_score(*args, _ptr(targets), _ptr(nll), _ptr(pred), rows, n_classes,
+                                                _ptr(out_row_map), _stream()))
+        return score
     if out16 is not None:
         with _Prof("head", rows * n_classes * (4 * k + 2)):
-            check(_native.lib().nnam_head_f16(ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb),
-                                              _ptr(rlb), _ptr(prior), float(prior_scale), int(bool(final_normalize)),
-                                              _ptr(o16), o16.stride(0), _ptr(ref), rows, n_classes, _ptr(out_row_map),
-                                              _stream()))
+            check(_native.lib().nnam_head_f16(*args, _ptr(o16), o16.stride(0), _ptr(ref), rows, n_classes,
+                                              _ptr(out_row_map), _stream()))
         return out16
     with _Prof("head", rows * n_classes * 4 * (k + 1)):
         if out_row_map is None:
-            check(_native.lib().nnam_head(ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb),
-                                          _ptr(rlb), _ptr(prior), float(prior_scale), int(bool(final_normalize)),
-                                          _ptr(out), out.stride(0), rows, n_classes, _stream()))
+            check(_native.lib().nnam_head(*args, _ptr(out), out.stride(0), rows, n_classes, _stream()))
         else:
-            check(_native.lib().nnam_head_scatter(ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb),
-                                                  _ptr(rlb), _ptr(prior), float(prior_scale),
-                                                  int(bool(final_normalize)), _ptr(out), out.stride(0), rows,
-                                                  n_classes, _ptr(out_row_map), _stream()))
+            check(_native.lib().nnam_head_scatter(*args, _ptr(out), out.stride(0), rows, n_classes, _ptr(out_row_map),
+                                                  _stream()))
     return out
-
-
-def head_score(logits, n_classes, targets, nll, pred, rows=None, weights=None, pre_normalize=False, rpl=None, prior=None,
-               prior_scale=1.0, final_normalize=True, out_row_map=None):
-    """K4 scored against frame targets (nnam_head_score): the rows :func:`head` would write are reduced to nll[q] =
-    -y[q][targets[q]] (0 for target -1) and pred[q] = argmax_c y[q][c] (lowest column on ties); a zero-fill map entry
-    -2 - q gives nll 0, pred -1.  ``targets`` / ``nll`` / ``pred``: int32 / f32 / int32, indexed by output row."""
-    if isinstance(logits, torch.Tensor):
-        logits = [logits]
-    for t in logits:
-        _req(t, torch.float32, "logits")
-    ld_in = logits[0].stride(0)
-    if any(t.stride(0) != ld_in for t in logits):
-        raise NnamError("head: all inputs must share one leading dimension")
-    if rows is None:
-        rows = logits[0].shape[0]
-    targets, nll, pred = _req_score((targets, nll, pred))
-    k = len(logits)
-    ptrs = (ctypes.c_void_p * k)(*[t.data_ptr() for t in logits])
-    wts = None if weights is None else (ctypes.c_float * k)(*[float(w) for w in weights])
-    rw = rb = rlb = None
-    if rpl is not None:
-        rw, rb, rlb = rpl
-        for t in (rw, rb, rlb):
-            _req(t, torch.float32, "rpl")
-    _req(prior, torch.float32, "prior")
-    _req(out_row_map, torch.int32, "out_row_map")
-    with _Prof("head", rows * (n_classes * 4 * k + 12)):
-        check(_native.lib().nnam_head_score(ptrs, wts, k, ld_in, int(bool(pre_normalize)), _ptr(rw), _ptr(rb), _ptr(rlb),
-                                            _ptr(prior), float(prior_scale), int(bool(final_normalize)), _ptr(targets),
-                                            _ptr(nll), _ptr(pred), rows, n_classes, _ptr(out_row_map), _stream()))
-    return nll, pred
 
 
 def widen_f16_host(src16, row_ref, dst, threads=1, dst_rows=None):

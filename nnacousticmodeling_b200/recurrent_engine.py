@@ -716,14 +716,12 @@ def _phase_split(lens):
     return [np.sort(by_len[a:b]) for a, b in zip(bounds[:-1], bounds[1:])]
 
 
-def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, out_dev, timedelay, fix_timedelay_tail,
-                   nb, device, stepwise, out16=None, out_starts=None, score=None):
+def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, dest, timedelay, fix_timedelay_tail,
+                   nb, device, stepwise, out_starts=None):
     """One subset of utterances (start frame relative to the shard and length of each) through the whole net:
-    packed gather -> layers -> output GEMM -> head, which scatters the rows into ``out_dev`` (all frames of the shard)
-    or, with ``out16`` = (fp16 rows, row maxima), into the compact transfer format (ops.head), or, with ``score`` =
-    device (targets, nll, pred) of all frames of the shard, scores them (ops.head_score).  ``out_starts``: first
-    OUTPUT row of every utterance when that differs from its first input frame (the compact format packs the rows of a
-    subset one after the other)."""
+    packed gather -> layers -> output GEMM -> head, which scatters the rows into the head destination ``dest`` (see
+    engine.run_head) over all frames of the shard.  ``out_starts``: first OUTPUT row of every utterance when that
+    differs from its first input frame (the compact format packs the rows of a subset one after the other)."""
     if out_starts is None:
         out_starts = starts
     plan = plans[0]
@@ -773,8 +771,6 @@ def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, o
     logits = []
     fused = fused_head_ok(models, head, plans[0].out.k)
     for k, (m, pl) in enumerate(zip(models, plans)):
-        if m.in_size != d_in or m.n_out != n_out:
-            raise NnamError("forward_utterances: ensemble members must share input and output sizes")
         key = (pl.cell, pl.hidden, pl.n_dirs)
         pl_stepwise = pl.cell == CELL_PEEPHOLE and not pl.peep_persistent
         if pl_stepwise != stepwise:
@@ -792,29 +788,9 @@ def _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, starts, lens, o
         pl.out(h_hi, h_lo, rows, "identity", OUT_F32, out=(lg, None))
         logits.append(lg)
     for u in np.nonzero(lens < timedelay)[0]:  # utterances shorter than the delay have rows no packed row maps to
-        r0, r1 = int(out_starts[u]), int(out_starts[u] + lens[u])
-        if score is not None:
-            score[1][r0:r1].zero_()
-            score[2][r0:r1].fill_(-1)
-            continue
-        for t in ((out_dev,) if out16 is None else out16):
-            t[r0:r1].zero_()
-    prior = _dev_vec(head.prior, device)
-    rpl = None if head.rpl is None else tuple(_dev_vec(head.rpl[k], device) for k in ("W", "b", "lb"))
-    if fused:
-        if score is not None:
-            plans[0].out.logsoftmax(h_hi, h_lo, rows, prior=prior, prior_scale=head.prior_scale, out_row_map=d_dst,
-                                    score=score)
-            return
-        plans[0].out.logsoftmax(h_hi, h_lo, rows, prior=prior, prior_scale=head.prior_scale, out_row_map=d_dst,
-                                out=None if out16 is not None else out_dev, out16=out16)
-        return
-    hkw = dict(rows=rows, weights=head.weights, pre_normalize=head.pre_normalize, rpl=rpl, prior=prior,
-               prior_scale=head.prior_scale, final_normalize=head.final_normalize, out_row_map=d_dst)
-    if score is not None:
-        ops.head_score(logits, n_out, *score, **hkw)
-        return
-    ops.head(logits, n_out, out=out_dev, out16=out16, **hkw)
+        engine.zero_rows(dest, int(out_starts[u]), int(out_starts[u] + lens[u]))
+    engine.run_head(head.device_args(device), dest, rows, out_row_map=d_dst, logits=logits, n_out=n_out,
+                    fused=plans[0].out if fused else None, h=(h_hi, h_lo))
 
 
 class _PackedDrainer:
@@ -827,20 +803,10 @@ class _PackedDrainer:
     def __init__(self, plan, out, out16, n_out, side, device, threads):
         import queue
         import threading
-        self.piece = max(256, int(os.environ.get("NNAM_PIECE_ROWS", "4096")))
-        self.slots = max(2, int(os.environ.get("NNAM_PIECE_SLOTS", "4")))
-        ld16 = out16[0].stride(0)
-        key = ("f16", self.piece, n_out, self.slots)
-        cache = plan.__dict__.setdefault("_stage", {})
-        if key not in cache:
-            cache.clear()
-            cache[key] = [(torch.empty((self.piece, ld16), dtype=torch.float16, pin_memory=True),
-                           torch.empty((self.piece,), dtype=torch.float32, pin_memory=True)) for _ in range(self.slots)]
-        self.stage = cache[key]
+        stage = engine.staging_ring(plan, True, max(256, int(os.environ.get("NNAM_PIECE_ROWS", "4096"))), n_out)
         out_np = out.numpy() if isinstance(out, torch.Tensor) else out
-        self.writer = engine._ChunkWriter(self.stage, True, out_np, None, n_out, threads)
+        self.writer = engine._ChunkWriter(stage, True, out_np, None, n_out, threads)
         self.out16, self.side, self.device = out16, side, device
-        self.k = 0
         self.err = None
         self.q = queue.Queue()
         self.thread = threading.Thread(target=self._run, name="nnam-drain", daemon=True)
@@ -864,19 +830,8 @@ class _PackedDrainer:
                 pass
 
     def _drain(self, done, p0, dst_rows):
-        side, stage, piece = self.side, self.stage, self.piece
-        side.wait_event(done)
-        for a0 in range(0, len(dst_rows), piece):
-            a1 = min(a0 + piece, len(dst_rows))
-            slot = self.k % self.slots
-            self.k += 1
-            self.writer.wait_free(slot)
-            with torch.cuda.stream(side):
-                stage[slot][0][:a1 - a0].copy_(self.out16[0][p0 + a0:p0 + a1], non_blocking=True)
-                stage[slot][1][:a1 - a0].copy_(self.out16[1][p0 + a0:p0 + a1], non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(side)
-            self.writer.submit(slot, 0, dst_rows[a0:a1], ev)
+        self.side.wait_event(done)
+        self.writer.ship(self.side, (self.out16[0][p0:], self.out16[1][p0:]), len(dst_rows), dst_rows)
 
     def close(self):
         self.q.put(None)
@@ -925,10 +880,9 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
         raise NnamError("forward_utterances: empty utterance in offsets")
     with torch.cuda.device(device):
         plans = [get_plan(m, device) for m in models]
+        engine.check_ensemble(models, plans, "forward_utterances: ")
         plan = plans[0]
         ws = plan.ws
-        if any(p.prec.spec != plan.prec.spec for p in plans):
-            raise NnamError("forward_utterances: all ensemble members must use the same precision mode")
         stepwise = plan.cell == CELL_PEEPHOLE and not plan.peep_persistent
 
         if isinstance(x, torch.Tensor) and x.is_cuda:
@@ -959,16 +913,16 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
             raise NnamError("forward_utterances: a scoring pass writes no rows (out must be None)")
         compact = (not on_dev and score is None) and engine.use_compact_transfer(plan, transfer, recurrent=True,
                                                                                  host_threads=host_threads)
-        out16 = sc_dev = None
         if score is not None:
             sc_dev = engine.score_buffers(ws, "rnn", score[0], f_lo, f_hi)
-            out_dev = None
+            dest = {"score": sc_dev}
         elif compact:
-            ld16 = round_up(n_out, 8)
-            out16 = (ws.get("rnn.out16", n_rows, ld16, torch.float16), ws.get("rnn.ref", n_rows, 1, torch.float32).view(-1))
-            out_dev = None
+            out16 = (ws.get("rnn.out16", n_rows, round_up(n_out, 8), torch.float16),
+                     ws.get("rnn.ref", n_rows, 1, torch.float32).view(-1))
+            dest = {"out16": out16}
         else:
             out_dev = out[f_lo:f_hi] if on_dev else ws.get("rnn.out", n_rows, n_out, torch.float32)
+            dest = {"out": out_dev}
         phases = [np.arange(len(lens))] if (on_dev or stepwise) else _phase_split(lens)
         main = torch.cuda.current_stream()
         side = None
@@ -983,9 +937,9 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
                 o_starts = None
                 if compact:
                     o_starts = packed + np.concatenate([[0], np.cumsum(p_lens[:-1])]).astype(np.int64)
-                _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, p_starts, p_lens, out_dev, timedelay,
-                               fix_timedelay_tail, nb, device, stepwise, out16=out16, out_starts=o_starts, score=sc_dev)
-                if on_dev or sc_dev is not None:
+                _forward_phase(models, plans, head, x_dev, iv_dev, add, mul, p_starts, p_lens, dest, timedelay,
+                               fix_timedelay_tail, nb, device, stepwise, out_starts=o_starts)
+                if on_dev or score is not None:
                     continue
                 out_host = None if compact else _as_host_tensor(out)
                 if len(phases) == 1 and not compact:
@@ -1019,7 +973,7 @@ def forward_utterances(model, x, offsets, out, u0, u1, ft=None, ivectors=None, t
         finally:
             if drainer is not None:  # an error above: let the helper thread go
                 drainer.abort()
-        if sc_dev is not None:
+        if score is not None:
             engine.download_scores(sc_dev, score, f_lo, f_hi)
         main.synchronize()
         if side is not None:

@@ -62,7 +62,7 @@ def _row_map(rng, rows, n_out):
 @pytest.mark.parametrize("c", [39, 1909, 2048])
 @pytest.mark.parametrize("case", ["one", "one_unaligned", "three", "three_prenorm", "rpl", "prior"])
 @pytest.mark.parametrize("mapped", [False, True])
-def test_head_score_matches_head_scatter(ops, c, case, mapped):
+def test_head_score_form_matches_head_scatter(ops, c, case, mapped):
     rng = np.random.default_rng(c + len(case))
     rows = 333
     k = 3 if case.startswith("three") else 1
@@ -86,7 +86,7 @@ def test_head_score_matches_head_scatter(ops, c, case, mapped):
     ops.head(logits, c, out=out, **kw)
     nll = torch.full((n_out,), SENT_NLL, device="cuda")
     pred = torch.full((n_out,), SENT_PRED, dtype=torch.int32, device="cuda")
-    ops.head_score(logits, c, _t(targets), nll, pred, **kw)
+    ops.head(logits, c, score=(_t(targets), nll, pred), **kw)
     torch.cuda.synchronize()
     _check_rows(out.cpu().numpy(), targets, nll.cpu().numpy(), pred.cpu().numpy(), written, zero)
 
