@@ -53,6 +53,9 @@ struct GemmParams {
   int f16;        // operands (and 16-bit outputs) are fp16 instead of bf16
   int act;        // NNAM_ACT_*
   const float* bias;
+  void* out_hi;   // output planes and leading dimension, for the direct stores of a row's ragged last box
+  void* out_lo;
+  long long ldo;
 };
 
 // barrier among the four epilogue warps only (named barrier 1, 128 threads)
@@ -82,12 +85,48 @@ __device__ __forceinline__ void apply_act(float (&v)[NV], int act) {  // warp-un
 
 // Output tile staging: the warp's 32 rows x 128 B go to shared memory in the SWIZZLE_128B pattern (16-byte chunk j of
 // row r lives at chunk position j ^ (r & 7): conflict-free for 8 consecutive lanes), then ONE lane hands the box to
-// the TMA store engine, which clips rows >= M and columns >= N.  Replaces per-thread row-strided global stores, whose
-// 32 separate lines per instruction had the L1/LSU pipe at ~73 % (profiles/r01_cfg2_gemm_before.md).
+// the TMA store engine, which clips rows >= M and columns >= N (the latter only at 16-byte granularity: see
+// box_crosses_ragged_end).  Replaces per-thread row-strided global stores, whose 32 separate lines per instruction
+// had the L1/LSU pipe at ~73 % (profiles/r01_cfg2_gemm_before.md).
 __device__ __forceinline__ void stage_row_128B(uint8_t* box, int lane, const uint4 (&chunks)[8]) {
   uint8_t* row = box + lane * 128;
 #pragma unroll
   for (int j = 0; j < 8; ++j) *reinterpret_cast<uint4*>(row + ((j ^ (lane & 7)) << 4)) = chunks[j];
+}
+
+// The TMA store clips a box that crosses column N only at 16-byte granularity: the rest of the 16-byte segment holding
+// column N - 1 would be written too.  When N does not end on a 16-byte boundary, the box that crosses N is therefore
+// stored by each lane for its own row, element by element, and nothing past column N is touched.
+template <int OUT_KIND>
+__device__ __forceinline__ bool box_crosses_ragged_end(int col, int n) {
+  constexpr int BOX_COLS = OUT_KIND == NNAM_OUT_F32 ? 32 : 64;
+  constexpr int PER_16B = OUT_KIND == NNAM_OUT_F32 ? 4 : 8;
+  return col + BOX_COLS > n && (n % PER_16B) != 0;
+}
+template <int OUT_KIND>
+__device__ __forceinline__ void store_row_prefix(void* base, long long ldo, int row, int col, int valid,
+                                                 const uint4 (&chunks)[8]) {
+  if (OUT_KIND == NNAM_OUT_F32) {
+    uint32_t* d = static_cast<uint32_t*>(base) + static_cast<long long>(row) * ldo + col;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const uint32_t w[4] = {chunks[j].x, chunks[j].y, chunks[j].z, chunks[j].w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e)
+        if (4 * j + e < valid) d[4 * j + e] = w[e];
+    }
+  } else {
+    uint16_t* d = static_cast<uint16_t*>(base) + static_cast<long long>(row) * ldo + col;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const uint32_t w[4] = {chunks[j].x, chunks[j].y, chunks[j].z, chunks[j].w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        if (8 * j + 2 * e < valid) d[8 * j + 2 * e] = static_cast<uint16_t>(w[e] & 0xffffu);
+        if (8 * j + 2 * e + 1 < valid) d[8 * j + 2 * e + 1] = static_cast<uint16_t>(w[e] >> 16);
+      }
+    }
+  }
 }
 
 // Registers are capped (not via __launch_bounds__, which would let ptxas take 240) so that a 256-thread GEMM CTA leaves
@@ -297,6 +336,11 @@ __global__ void __maxnreg__(GEMM_MAX_REGS)
             for (int j = 0; j < 8; ++j)
               chunks[j] = make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
                                      pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
+          }
+          if (box_crosses_ragged_end<OUT_KIND>(col, p.N)) {  // warp-uniform
+            if (row0 + lane < p.M) store_row_prefix<OUT_KIND>(o == 0 ? p.out_hi : p.out_lo, p.ldo, row0 + lane, col,
+                                                              p.N - col, chunks);
+            continue;
           }
           uint8_t* box = boxes + box_sel * EPI_BOX_BYTES;
           if (lane == 0) tma_store_wait_read<NBOX - 1>();  // the store issued from this box NBOX boxes ago has read it
@@ -549,6 +593,11 @@ __global__ void __cluster_dims__(2, 1, 1) __maxnreg__(GEMM_MAX_REGS)
               chunks[j] = make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
                                      pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
           }
+          if (box_crosses_ragged_end<OUT_KIND>(col, p.N)) {  // warp-uniform
+            if (row0 + lane < p.M) store_row_prefix<OUT_KIND>(o == 0 ? p.out_hi : p.out_lo, p.ldo, row0 + lane, col,
+                                                              p.N - col, chunks);
+            continue;
+          }
           uint8_t* box = boxes + box_sel * EPI_BOX_BYTES;
           if (lane == 0) tma_store_wait_read<1>();
           __syncwarp();
@@ -697,6 +746,9 @@ int gemm_bias_act(const void* a_hi, const void* a_lo, long long lda, const void*
   p.f16 = elem == NNAM_ELEM_F16;
   p.act = act;
   p.bias = bias;
+  p.out_hi = out_hi;
+  p.out_lo = out_lo;
+  p.ldo = ldo;
 
   // tm[0..3] = A hi/lo, W hi/lo (loads); tm[4..5] = output hi/lo (stores: 32-row x 128-byte boxes, clipped at M x N)
   CUtensorMap tm[6];

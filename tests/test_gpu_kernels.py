@@ -246,8 +246,10 @@ def test_linear_logsoftmax_fused(ops, dev, m, n, k, elem, nsplit):
 
 @pytest.mark.parametrize("m,n,k", [(128, 256, 64), (1, 16, 8), (300, 1024, 544), (1000, 1909, 440), (77, 40, 40),
                                    (2048, 2048, 2048), (513, 2048, 140), (129, 1909, 1024),
-                                   # M >= 4096 runs the CTA-pair (cta_group::2) kernel: ragged M, ragged N, short K
-                                   (4096, 2048, 2048), (4173, 1909, 1024), (5000, 512, 544), (4100, 128, 72)])
+                                   # M >= 4096 with K >= 384 runs the CTA-pair (cta_group::2) kernel: ragged M, ragged N
+                                   (4096, 2048, 2048), (4173, 1909, 1024), (5000, 512, 544),
+                                   # single-CTA kernel at large M: K = 72 < 384 keeps it off the pair kernel
+                                   (4100, 128, 72)])
 @pytest.mark.parametrize("mode", ["bf16", "fp32"])
 def test_linear_bias_act(ops, dev, m, n, k, mode):
     rng = np.random.default_rng(m * 7 + n)
